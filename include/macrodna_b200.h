@@ -287,6 +287,26 @@ int mcd_subinstance_steps(mcd_handle h, const int32_t* rna_rows, int64_t m_sub, 
 int mcd_subinstance_sweep(mcd_handle h, int64_t nrep, const int32_t* rna_rows, int64_t m_sub, const int32_t* dna_cols,
                           int64_t n_sub, int32_t* assign, int32_t* step, double* step_obj, double* cert_gap,
                           int concurrency, mcd_stats* stats);
+/*
+ * mcd_loo_sweep: the reference's leave-one-out experiment (run_loo_experiment.py:201-319), `ncells` replicates in one
+ * call on the resident M x N matrix, kept `concurrency` at a time in flight like mcd_subinstance_sweep.  Replicate r
+ * leaves out RNA row q = cells[r] (HOST int32 in [0, M); repeats allowed):
+ *   - the step loop runs on C with row q deleted (the M-1 other rows in ascending order, `np.delete(corrs, q, 0)`,
+ *     all N columns; mcd_num_steps(M-1, N) steps); M == 1 leaves an empty replicate and no solve runs;
+ *   - q takes the column of highest C[q, j] among those matched at most k_steps - 1 times by the replicate (:296-309);
+ *     among exact ties the highest column index (the order a stable ascending sort, reversed, visits);
+ *   - total = the step objectives, then the test cell's correlation if a column was found, summed in FP64 exactly as
+ *     the reference's `float(sum(obj_scores))` sums them under CPython >= 3.12 (first term added to 0, the rest with
+ *     Neumaier's compensation), so that it is bit-equal to the total of MaCroDNA.leave_one_out.
+ * Required HOST outputs [ncells]: test_col (-1 if no column is eligible), test_corr (0 then), total.  Optional HOST
+ * outputs (NULL to skip; a whole-biopsy sweep need not move O(M^2) data): assign / step [ncells, M-1], step_obj
+ * [ncells, nsteps], match_corr [ncells, M-1] = C[row, assign] (the `corr_val` column), cert_gap [ncells] = the
+ * replicate's largest per-step relative duality gap.  stats as mcd_subinstance_sweep fills it.
+ * Measured throughput: not measured yet (see DESIGN.md section 5b).
+ */
+int mcd_loo_sweep(mcd_handle h, const int32_t* cells, int64_t ncells, int64_t k_steps, int32_t* test_col,
+                  double* test_corr, double* total, int32_t* assign, int32_t* step, double* step_obj, double* match_corr,
+                  double* cert_gap, int concurrency, mcd_stats* stats);
 int mcd_corr_rows(mcd_handle h, const int32_t* rows, int64_t nrows, double* out, int out_space);
 /* out[k] = C[rows[k], cols[k]] of the resident matrix (HOST indices, HOST out): the `corr_val` of a sub-instance's
  * matched pairs (run_loo_experiment.py:285). */

@@ -99,6 +99,7 @@ SIGNATURES = {
     "mcd_lap_certify": (_I, [_VP, _VP, _I64, _I64, _I64, _VP, _VP, _VP]),
     "mcd_subinstance_steps": (_I, [_VP, _VP, _I64, _VP, _I64, _VP, _VP, _VP, _I, C.POINTER(McdStats)]),
     "mcd_subinstance_sweep": (_I, [_VP, _I64, _VP, _I64, _VP, _I64, _VP, _VP, _VP, _VP, _I, C.POINTER(McdStats)]),
+    "mcd_loo_sweep": (_I, [_VP, _VP, _I64, _I64, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _I, C.POINTER(McdStats)]),
     "mcd_corr_rows": (_I, [_VP, _VP, _I64, _VP, _I]),
     "mcd_corr_pairs": (_I, [_VP, _VP, _VP, _I64, _VP]),
     "mcd_null_assignments": (_I, [_VP, _I64, C.c_uint64, _VP, _VP, _I]),
@@ -343,6 +344,26 @@ class Handle:
         self.check(self.lib.mcd_subinstance_sweep(self.h, nrep, _ptr(rna_rows), m, _ptr(dna_cols), n, _ptr(assign),
                                                   _ptr(step), _ptr(objs), _ptr(gaps), int(concurrency), C.byref(stats)))
         return assign, step, objs, gaps, stats
+
+    def loo_sweep(self, cells, k_steps, M, N, full=False, concurrency=8):
+        """Leave-one-out replicates of the resident M x N matrix, one per entry of ``cells`` (``mcd_loo_sweep``).
+        Returns (dict of arrays, stats): ``test_col`` [ncells] (-1: no eligible column), ``test_corr``, ``total``,
+        ``cert_gap``; with ``full`` also ``assign`` / ``step`` / ``match_corr`` [ncells, M-1] and ``step_obj``
+        [ncells, nsteps]."""
+        cells = np.ascontiguousarray(cells, dtype=np.int32).ravel()
+        n, m = cells.size, int(M) - 1
+        nsteps = self.lib.mcd_num_steps(m, int(N))
+        out = {"test_col": np.empty(n, dtype=np.int32), "test_corr": np.empty(n, dtype=np.float64),
+               "total": np.empty(n, dtype=np.float64), "cert_gap": np.empty(n, dtype=np.float64)}
+        if full:
+            out.update(assign=np.empty((n, m), dtype=np.int32), step=np.empty((n, m), dtype=np.int32),
+                       step_obj=np.empty((n, nsteps), dtype=np.float64), match_corr=np.empty((n, m), dtype=np.float64))
+        stats = McdStats()
+        self.check(self.lib.mcd_loo_sweep(self.h, _ptr(cells), n, int(k_steps), _ptr(out["test_col"]),
+                                          _ptr(out["test_corr"]), _ptr(out["total"]), _ptr(out.get("assign")),
+                                          _ptr(out.get("step")), _ptr(out.get("step_obj")), _ptr(out.get("match_corr")),
+                                          _ptr(out["cert_gap"]), int(concurrency), C.byref(stats)))
+        return out, stats
 
     def corr_rows(self, rows, N):
         rows = np.ascontiguousarray(rows, dtype=np.int32)

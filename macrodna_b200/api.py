@@ -118,6 +118,7 @@ class MaCroDNA:
         self.last_objective = None  # per-step objective (the `m.objVal` of each reference `ilp` call)
         self.last_assign = None     # int32 DNA column per RNA cell
         self.last_step = None       # int32 1-based step per RNA cell
+        self.last_loo = None        # leave_one_out_sweep: left-out cells, certificate gaps, stats
 
     # -- the frames.  The reference overwrites self.rna_df / self.dna_df with the gene-filtered frames
     #    (macrodna.py:90-91).  Here the filtering of the DATA happens on the device (index gather in K1), so the
@@ -348,36 +349,89 @@ class MaCroDNA:
         if not 0 <= cell_idx < M:
             raise IndexError("pop index out of range")  # rna_cells.pop(cell_idx), :206
         rows = np.delete(np.arange(M, dtype=np.int32), cell_idx)
-        rest = [c for k, c in enumerate(rna_cells) if k != cell_idx]
-        obj_scores = []
         if rows.size:
             assign, step, objs, _ = h.subinstance(rows, None, M=M, N=N)
             vals = h.corr_pairs(rows, assign)
-            obj_scores = [float(o) for o in objs]
         else:
             assign = np.empty(0, dtype=np.int32)
             step = np.empty(0, dtype=np.int32)
-            vals = np.empty(0)
-        res_dna = [dna_cells[j] for j in assign.tolist()]
-        res_rna = list(rest)
-        res_tag = step.tolist()
-        res_val = vals.tolist()
+            objs = vals = np.empty(0)
         cell_corr = h.corr_rows([cell_idx], N)[0]                     # np.take(corrs, cell_idx, axis=0), :226
         cnt = np.bincount(assign, minlength=N)                       # np.count_nonzero(tagged, axis=0), :296
         eligible = cnt <= (K_steps - 1)                              # :298
+        test_col, test_corr = -1, 0.0
         for idx_ in np.argsort(cell_corr)[::-1]:                     # :300-309
             if eligible[idx_]:
-                res_dna.append(dna_cells[idx_])
-                res_rna.append(rna_cells[cell_idx])
-                res_tag.append("TEST")
-                obj_scores.append(float(cell_corr[idx_]))
-                res_val.append(float(cell_corr[idx_]))
+                test_col, test_corr = int(idx_), float(cell_corr[idx_])
                 break
+        return self._loo_frame(cell_idx, assign, step, vals, objs, test_col, test_corr, biopsy_name)
+
+    def _loo_frame(self, cell_idx, assign, step, vals, objs, test_col, test_corr, biopsy_name):
+        """The ``(tagged, objective)`` of one leave-one-out replicate (run_loo_experiment.py:246-319): the remaining
+        cells with their DNA cell, step and matched correlation, then the left-out cell's ``"TEST"`` row if a DNA
+        cell was eligible (``test_col >= 0``); the objective is ``float(sum(obj_scores))`` in the reference's order."""
+        rna_cells, dna_cells = self._resident_cells
+        res_dna = [dna_cells[j] for j in assign.tolist()]
+        res_rna = [c for k, c in enumerate(rna_cells) if k != cell_idx]
+        res_tag = step.tolist()
+        res_val = vals.tolist()
+        obj_scores = [float(o) for o in objs]
+        if test_col >= 0:
+            res_dna.append(dna_cells[test_col])
+            res_rna.append(rna_cells[cell_idx])
+            res_tag.append("TEST")
+            obj_scores.append(test_corr)
+            res_val.append(test_corr)
         tagged = pd.DataFrame(list(zip(res_dna, res_rna, res_tag, res_val)),
                               columns=["predicted_dna_cell", "rna_cell", "step", "corr_val"]).set_index("rna_cell")
         if self.verbose:
             print("name of the left-out RNA cell %s from sample %s" % (rna_cells[cell_idx], biopsy_name))
         return tagged, float(sum(obj_scores))
+
+    def leave_one_out_sweep(self, cell_idx=None, K_steps=None, biopsy_name=None, frames=False, concurrency=8):
+        """Every leave-one-out replicate of ``cell_idx`` (positions as in :meth:`leave_one_out`; None = every RNA
+        cell) in one call (``mcd_loo_sweep``): the solves are kept ``concurrency`` at a time in flight on the GPU.
+        ``K_steps`` defaults to ``ceil(M / N)``, what run_loo_experiment.py passes.
+
+        Returns a frame indexed by ``rna_cell`` (the left-out cells, in ``cell_idx`` order) with columns
+        ``predicted_dna_cell`` (None when no DNA cell is eligible), ``corr_val`` and ``objective``; per-replicate
+        certificate gaps and the stats go to ``self.last_loo``.  ``frames=True`` returns instead the list of
+        ``(tagged, objective)`` a loop of ``leave_one_out(q, K_steps, biopsy_name)`` returns."""
+        if self._rna_df is None or self._dna_df is None:
+            raise ValueError("rna_df and dna_df are required")
+        M, N = len(self._rna_df.columns), len(self._dna_df.columns)
+        cells = list(range(M)) if cell_idx is None else [int(q) for q in cell_idx]
+        if not cells:
+            raise ValueError("cell_idx is empty")
+        for q in cells:
+            if not 0 <= q < M:
+                raise IndexError("pop index out of range")  # rna_cells.pop(cell_idx), run_loo_experiment.py:206
+        if K_steps is None:
+            K_steps = -(-M // N) if N else 1
+        K_steps = int(K_steps)
+        if K_steps < 1:
+            raise ValueError("K_steps must be >= 1")
+        dna_cells = list(self._dna_df.columns)
+        if len(set(dna_cells)) != len(dna_cells) and \
+                self._duplicate_dna_cells(dna_cells, self._cells_by_genes(self._dna_df)) is not None:
+            raise ValueError("leave_one_out_sweep: the DNA frame repeats cells with identical data (a resampled frame); "
+                             "its correlation matrix is computed on the distinct cells, so leave-one-out replicates "
+                             "cannot be taken from it -- pass the frame of distinct DNA cells")
+        h = self._ensure_resident()
+        rna_cells, dna_cells = self._resident_cells
+        M, N = self._resident_shape
+        res, stats = h.loo_sweep(cells, K_steps, M, N, full=frames, concurrency=concurrency)
+        self.last_loo = {"cells": np.asarray(cells), "cert_gap": res["cert_gap"], "stats": stats.as_dict()}
+        if frames:
+            return [self._loo_frame(q, res["assign"][r], res["step"][r], res["match_corr"][r], res["step_obj"][r],
+                                    int(res["test_col"][r]), float(res["test_corr"][r]), biopsy_name)
+                    for r, q in enumerate(cells)]
+        if self.verbose:
+            for q in cells:
+                print("name of the left-out RNA cell %s from sample %s" % (rna_cells[q], biopsy_name))
+        pred = [dna_cells[j] if j >= 0 else None for j in res["test_col"].tolist()]
+        return pd.DataFrame({"predicted_dna_cell": pred, "corr_val": res["test_corr"], "objective": res["total"]},
+                            index=pd.Index([rna_cells[q] for q in cells], name="rna_cell"))
 
     def cell2clone_assignment(self):
         """macrodna.py:188-199: cell2cell + ``dna_label.set_index("cell").loc[predict_cell]["clone"]``."""

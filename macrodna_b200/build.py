@@ -13,7 +13,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libmacrodna_b200.so")
-SOURCES = ["api.cu", "standardize.cu", "corr_fp64.cu", "corr_tc.cu", "corr_ozaki.cu", "lap.cu", "null_test.cu", "stage.cu"]
+SOURCES = ["api.cu", "standardize.cu", "corr_fp64.cu", "corr_tc.cu", "corr_ozaki.cu", "lap.cu", "null_test.cu", "loo.cu", "stage.cu"]
 HEADERS = ["mcd_internal.cuh", os.path.join("..", "..", "include", "macrodna_b200.h")]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 

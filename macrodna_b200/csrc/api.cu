@@ -6,6 +6,7 @@
 #include <chrono>
 #include <cstddef>
 #include <cstring>
+#include <functional>
 #include <new>
 #include <thread>
 
@@ -1457,41 +1458,56 @@ static int sweep_worker(mcd_context* h, size_t k, mcd_context** out) {
   return MCD_OK;
 }
 
-int mcd_subinstance_sweep(mcd_handle h, int64_t nrep, const int32_t* rna_rows, int64_t m_sub, const int32_t* dna_cols,
-                          int64_t n_sub, int32_t* assign, int32_t* step, double* step_obj, double* cert_gap,
-                          int concurrency, mcd_stats* stats) {
-  if (!h) return MCD_ERR_INVALID;
-  if (!assign || !step || !dna_cols || nrep < 1 || m_sub < 1 || n_sub < 1 || h->last_M < 1 || h->last_assign == nullptr)
-    return mcd_fail(h, MCD_ERR_INVALID, "mcd_subinstance_sweep: no mcd_cell2cell result is resident / bad arguments");
-  if (!rna_rows && m_sub != h->last_M)
-    return mcd_fail(h, MCD_ERR_INVALID, "mcd_subinstance_sweep: NULL rna_rows means all rows");
-  for (int64_t i = 0; rna_rows && i < m_sub; ++i)
-    if (rna_rows[i] < 0 || rna_rows[i] >= h->last_M)
-      return mcd_fail(h, MCD_ERR_INVALID, "mcd_subinstance_sweep: RNA row out of range");
-  for (int64_t j = 0; j < nrep * n_sub; ++j)
-    if (dna_cols[j] < 0 || dna_cols[j] >= h->last_N)
-      return mcd_fail(h, MCD_ERR_INVALID, "mcd_subinstance_sweep: DNA column out of range");
-  MCD_CUDA(h, cudaSetDevice(h->device));
-  int K = concurrency < 1 ? 8 : concurrency;
-  if (K > 32) K = 32;
-  if ((int64_t)K > nrep) K = (int)nrep;
-  const int64_t nsteps = mcd_num_steps(m_sub, n_sub);
-  const size_t rep_bytes = (step_out_bytes(m_sub, nsteps) + 255) / 256 * 256;
-  int64_t batch = (int64_t)((size_t)1 << 30) / (int64_t)rep_bytes;  // <= 1 GiB of per-replicate outputs at a time
-  if (batch < K) batch = K;
-  if (batch > nrep) batch = nrep;
+// The replicate sweep engine shared by mcd_subinstance_sweep and mcd_loo_sweep.  Replicates are independent step
+// loops of one shape (m_sub rows, n_sub columns); what makes one replicate differ from the next comes in as hooks.
+struct SweepPlan {
+  int K;              // worker contexts (replicates in flight)
+  int64_t nsteps;     // steps of every replicate
+  int64_t batch;      // replicates per batch
+  size_t step_bytes;  // the replicate's StepOut block (256-byte aligned)
+  size_t rep_bytes;   // step_bytes + the caller's extra bytes per replicate
+};
+
+static SweepPlan sweep_plan(int64_t nrep, int64_t m_sub, int64_t n_sub, size_t extra_rep_bytes, int concurrency) {
+  SweepPlan p;
+  p.K = concurrency < 1 ? 8 : concurrency;
+  if (p.K > 32) p.K = 32;
+  if ((int64_t)p.K > nrep) p.K = (int)nrep;
+  p.nsteps = mcd_num_steps(m_sub, n_sub);
+  p.step_bytes = (step_out_bytes(m_sub, p.nsteps) + 255) / 256 * 256;
+  p.rep_bytes = p.step_bytes + (extra_rep_bytes + 255) / 256 * 256;
+  p.batch = (int64_t)((size_t)1 << 30) / (int64_t)p.rep_bytes;  // <= 1 GiB of per-replicate outputs at a time
+  if (p.batch < p.K) p.batch = p.K;
+  if (p.batch > nrep) p.batch = nrep;
+  return p;
+}
+
+struct SweepHooks {
+  // on h->stream before the replicates of the batch [r0, r0 + nb) are dealt (uploads of the batch's indices); optional
+  std::function<int(int64_t r0, int64_t nb)> prepare;
+  // on worker w's stream, from w's host thread: cost block subC [m_sub, lds] and its transpose subCt [n_sub, ldst] of
+  // replicate r0 + b; *dna_class = DEVICE classes of duplicated DNA cells (see enqueue_step_loop) or NULL
+  std::function<int(mcd_context* w, int64_t r0, int64_t b, double* subC, int64_t lds, double* subCt, int64_t ldst,
+                    const int** dna_class)>
+      build;
+  // on h->stream after the workers joined, before the outputs go to the host: replicate b of the batch has its block
+  // at out + b * rep_bytes (StepOut first, the caller's extra bytes from step_bytes on); optional
+  std::function<int(int64_t r0, int64_t nb, char* out)> after;
+  // on the host once the batch synchronised, per replicate r = r0 + b: status bits and certificate gap in / out (a
+  // replicate may be solved again); optional
+  std::function<int(int64_t r, int64_t b, int& bad, double& gap)> redo;
+};
+
+static int sweep_replicates(mcd_context* h, const SweepPlan& P, int64_t nrep, int64_t m_sub, int64_t n_sub,
+                            int32_t* assign, int32_t* step, double* step_obj, double* cert_gap, mcd_stats* stats,
+                            const SweepHooks& hk) {
+  const int K = P.K;
+  const int64_t nsteps = P.nsteps, batch = P.batch;
+  const size_t rep_bytes = P.rep_bytes;
   int st;
-  void *p_idx = nullptr, *p_out = nullptr;
-  if ((st = mcd_ws(h, WS_SWEEP_IDX, (size_t)(m_sub + 2 * batch * n_sub) * 4, &p_idx))) return st;
+  void* p_out = nullptr;
   if ((st = mcd_ws(h, WS_SWEEP_OUT, (size_t)batch * rep_bytes, &p_out))) return st;
-  int* d_rows = rna_rows ? static_cast<int*>(p_idx) : nullptr;
-  int* d_cols = static_cast<int*>(p_idx) + m_sub;
-  int* d_clss = d_cols + batch * n_sub;
-  std::vector<int> clss((size_t)(batch * n_sub)), cls1;
-  std::vector<int64_t> n_extra((size_t)batch);
-  if (rna_rows) MCD_CUDA(h, cudaMemcpyAsync(d_rows, rna_rows, (size_t)m_sub * 4, cudaMemcpyHostToDevice, h->stream));
   const int64_t lds = (n_sub + 1) & ~1LL, ldst = (m_sub + 1) & ~1LL;
-  const double* C = static_cast<const double*>(h->ws[WS_C].ptr);
   // every worker solves on a slice of the chip: the cooperative grid of the wide rounds is capped so that K of them
   // are co-resident (the narrow rounds run on one 8- or 16-CTA cluster per solve anyway)
   std::vector<mcd_context*> ws((size_t)K);
@@ -1516,12 +1532,7 @@ int mcd_subinstance_sweep(mcd_handle h, int64_t nrep, const int32_t* rna_rows, i
   double host_enqueue_ms = 0.0;  // wall time of the enqueuing phase of every batch: reported as ms_h2d
   for (int64_t r0 = 0; r0 < nrep; r0 += batch) {
     const int64_t nb = nrep - r0 < batch ? nrep - r0 : batch;
-    MCD_CUDA(h, cudaMemcpyAsync(d_cols, dna_cols + r0 * n_sub, (size_t)nb * n_sub * 4, cudaMemcpyHostToDevice, h->stream));
-    for (int64_t b = 0; b < nb; ++b) {
-      n_extra[(size_t)b] = duplicate_classes(dna_cols + (r0 + b) * n_sub, n_sub, cls1);
-      std::copy(cls1.begin(), cls1.end(), clss.begin() + b * n_sub);
-    }
-    MCD_CUDA(h, cudaMemcpyAsync(d_clss, clss.data(), (size_t)nb * n_sub * 4, cudaMemcpyHostToDevice, h->stream));
+    if (hk.prepare && (st = hk.prepare(r0, nb))) return st;
     MCD_CUDA(h, cudaEventRecord(get_event(h, 5), h->stream));
     for (int k = 0; k < K; ++k) MCD_CUDA(h, cudaStreamWaitEvent(ws[k]->stream, get_event(h, 5), 0));
     // Replicates differ a lot in cost (a resampled replicate with a starved clone needs 10x the rounds of a balanced
@@ -1552,17 +1563,10 @@ int mcd_subinstance_sweep(mcd_handle h, int64_t nrep, const int32_t* rna_rows, i
         }
         double* subC = static_cast<double*>(pc);
         double* subCt = static_cast<double*>(pct);
-        dim3 grid((unsigned)((n_sub + 1023) / 1024 < 64 ? (n_sub + 1023) / 1024 : 64), grid_rows(m_sub));
-        gather_sub_kernel<<<grid, 256, 0, w->stream>>>(C, h->last_ldc, d_rows, d_cols + b * n_sub, m_sub, n_sub, subC, lds);
-        w->launches++;
-        if (cudaGetLastError() != cudaSuccess) {
-          wstatus[(size_t)k] = mcd_fail(w, MCD_ERR_CUDA, "gather_sub_kernel");
-          return;
-        }
+        const int* dna_class = nullptr;
         const StepOut out = carve_step_out(static_cast<char*>(p_out) + (size_t)b * rep_bytes, m_sub, nsteps);
-        if ((stw = mcd_transpose_f64(w, subC, m_sub, n_sub, lds, subCt, ldst)) ||
-            (stw = enqueue_step_loop(w, subC, lds, subCt, ldst, m_sub, n_sub, out, 0, false, false,
-                                     n_extra[(size_t)b] > 0 ? d_clss + b * n_sub : nullptr))) {
+        if ((stw = hk.build(w, r0, b, subC, lds, subCt, ldst, &dna_class)) ||
+            (stw = enqueue_step_loop(w, subC, lds, subCt, ldst, m_sub, n_sub, out, 0, false, false, dna_class))) {
           wstatus[(size_t)k] = stw;
           return;
         }
@@ -1588,12 +1592,15 @@ int mcd_subinstance_sweep(mcd_handle h, int64_t nrep, const int32_t* rna_rows, i
       MCD_CUDA(h, cudaEventRecord(get_event(ws[k], 0), ws[k]->stream));
       MCD_CUDA(h, cudaStreamWaitEvent(h->stream, get_event(ws[k], 0), 0));
     }
+    if (hk.after && (st = hk.after(r0, nb, static_cast<char*>(p_out)))) return st;
     // results of the batch: strided device block -> dense host arrays
     const StepOut o0 = carve_step_out(p_out, m_sub, nsteps);
-    MCD_CUDA(h, cudaMemcpy2DAsync(assign + r0 * m_sub, (size_t)m_sub * 4, o0.assign, rep_bytes, (size_t)m_sub * 4, (size_t)nb,
-                                  cudaMemcpyDeviceToHost, h->stream));
-    MCD_CUDA(h, cudaMemcpy2DAsync(step + r0 * m_sub, (size_t)m_sub * 4, o0.step, rep_bytes, (size_t)m_sub * 4, (size_t)nb,
-                                  cudaMemcpyDeviceToHost, h->stream));
+    if (assign)
+      MCD_CUDA(h, cudaMemcpy2DAsync(assign + r0 * m_sub, (size_t)m_sub * 4, o0.assign, rep_bytes, (size_t)m_sub * 4,
+                                    (size_t)nb, cudaMemcpyDeviceToHost, h->stream));
+    if (step)
+      MCD_CUDA(h, cudaMemcpy2DAsync(step + r0 * m_sub, (size_t)m_sub * 4, o0.step, rep_bytes, (size_t)m_sub * 4,
+                                    (size_t)nb, cudaMemcpyDeviceToHost, h->stream));
     if (step_obj)
       MCD_CUDA(h, cudaMemcpy2DAsync(step_obj + r0 * nsteps, (size_t)nsteps * 8, o0.obj, rep_bytes, (size_t)nsteps * 8,
                                     (size_t)nb, cudaMemcpyDeviceToHost, h->stream));
@@ -1607,19 +1614,7 @@ int mcd_subinstance_sweep(mcd_handle h, int64_t nrep, const int32_t* rna_rows, i
       int bad_b = fold_step_records(h, m_sub, n_sub, nsteps, hc.data() + b * nsteps, rc, stats, 0, false);
       double g = 0.0;
       for (int64_t s2 = 0; s2 < nsteps; ++s2) g = rc[s2].rel_gap > g ? rc[s2].rel_gap : g;
-      if ((bad_b & 2) && n_extra[(size_t)b] > 0) {
-        // certificate failed with the class treatment of duplicated cells: solve this replicate again without it
-        // (see mcd_subinstance_steps)
-        mcd_stats st2;
-        const int r = (int)(r0 + b);
-        const int rc2 = subinstance_steps_impl(h, rna_rows, m_sub, dna_cols + (int64_t)r * n_sub, n_sub,
-                                               assign + (int64_t)r * m_sub, step + (int64_t)r * m_sub,
-                                               step_obj ? step_obj + (int64_t)r * nsteps : nullptr, MCD_MEM_HOST, &st2, false,
-                                               &bad_b);
-        if (rc2 != MCD_OK && rc2 != MCD_ERR_NOT_CONVERGED) return rc2;
-        g = st2.cert_rel_gap;
-        if (stats) stats->sweep_fallbacks += 1;
-      }
+      if (hk.redo && (st = hk.redo(r0 + b, b, bad_b, g))) return st;
       bad |= bad_b;
       if (cert_gap) cert_gap[r0 + b] = h->opt.certify ? g : -1.0;
     }
@@ -1638,6 +1633,158 @@ int mcd_subinstance_sweep(mcd_handle h, int64_t nrep, const int32_t* rna_rows, i
     stats->kernel_launches = launches;
   }
   return step_status(h, bad);
+}
+
+int mcd_subinstance_sweep(mcd_handle h, int64_t nrep, const int32_t* rna_rows, int64_t m_sub, const int32_t* dna_cols,
+                          int64_t n_sub, int32_t* assign, int32_t* step, double* step_obj, double* cert_gap,
+                          int concurrency, mcd_stats* stats) {
+  if (!h) return MCD_ERR_INVALID;
+  if (!assign || !step || !dna_cols || nrep < 1 || m_sub < 1 || n_sub < 1 || h->last_M < 1 || h->last_assign == nullptr)
+    return mcd_fail(h, MCD_ERR_INVALID, "mcd_subinstance_sweep: no mcd_cell2cell result is resident / bad arguments");
+  if (!rna_rows && m_sub != h->last_M)
+    return mcd_fail(h, MCD_ERR_INVALID, "mcd_subinstance_sweep: NULL rna_rows means all rows");
+  for (int64_t i = 0; rna_rows && i < m_sub; ++i)
+    if (rna_rows[i] < 0 || rna_rows[i] >= h->last_M)
+      return mcd_fail(h, MCD_ERR_INVALID, "mcd_subinstance_sweep: RNA row out of range");
+  for (int64_t j = 0; j < nrep * n_sub; ++j)
+    if (dna_cols[j] < 0 || dna_cols[j] >= h->last_N)
+      return mcd_fail(h, MCD_ERR_INVALID, "mcd_subinstance_sweep: DNA column out of range");
+  MCD_CUDA(h, cudaSetDevice(h->device));
+  const SweepPlan P = sweep_plan(nrep, m_sub, n_sub, 0, concurrency);
+  const int64_t batch = P.batch, nsteps = P.nsteps;
+  int st;
+  void* p_idx = nullptr;
+  if ((st = mcd_ws(h, WS_SWEEP_IDX, (size_t)(m_sub + 2 * batch * n_sub) * 4, &p_idx))) return st;
+  int* d_rows = rna_rows ? static_cast<int*>(p_idx) : nullptr;
+  int* d_cols = static_cast<int*>(p_idx) + m_sub;
+  int* d_clss = d_cols + batch * n_sub;
+  std::vector<int> clss((size_t)(batch * n_sub)), cls1;
+  std::vector<int64_t> n_extra((size_t)batch);
+  if (rna_rows) MCD_CUDA(h, cudaMemcpyAsync(d_rows, rna_rows, (size_t)m_sub * 4, cudaMemcpyHostToDevice, h->stream));
+  const double* C = static_cast<const double*>(h->ws[WS_C].ptr);
+  SweepHooks hk;
+  hk.prepare = [&](int64_t r0, int64_t nb) -> int {
+    MCD_CUDA(h, cudaMemcpyAsync(d_cols, dna_cols + r0 * n_sub, (size_t)nb * n_sub * 4, cudaMemcpyHostToDevice, h->stream));
+    for (int64_t b = 0; b < nb; ++b) {
+      n_extra[(size_t)b] = duplicate_classes(dna_cols + (r0 + b) * n_sub, n_sub, cls1);
+      std::copy(cls1.begin(), cls1.end(), clss.begin() + b * n_sub);
+    }
+    MCD_CUDA(h, cudaMemcpyAsync(d_clss, clss.data(), (size_t)nb * n_sub * 4, cudaMemcpyHostToDevice, h->stream));
+    return MCD_OK;
+  };
+  hk.build = [&](mcd_context* w, int64_t, int64_t b, double* subC, int64_t lds, double* subCt, int64_t ldst,
+                 const int** dna_class) -> int {
+    dim3 grid((unsigned)((n_sub + 1023) / 1024 < 64 ? (n_sub + 1023) / 1024 : 64), grid_rows(m_sub));
+    gather_sub_kernel<<<grid, 256, 0, w->stream>>>(C, h->last_ldc, d_rows, d_cols + b * n_sub, m_sub, n_sub, subC, lds);
+    MCD_LAUNCH_CHECK(w, "gather_sub_kernel");
+    *dna_class = n_extra[(size_t)b] > 0 ? d_clss + b * n_sub : nullptr;
+    return mcd_transpose_f64(w, subC, m_sub, n_sub, lds, subCt, ldst);
+  };
+  hk.redo = [&](int64_t r, int64_t b, int& bad_b, double& g) -> int {
+    if (!((bad_b & 2) && n_extra[(size_t)b] > 0)) return MCD_OK;
+    // certificate failed with the class treatment of duplicated cells: solve this replicate again without it
+    // (see mcd_subinstance_steps)
+    mcd_stats st2;
+    const int rc2 = subinstance_steps_impl(h, rna_rows, m_sub, dna_cols + r * n_sub, n_sub, assign + r * m_sub,
+                                           step + r * m_sub, step_obj ? step_obj + r * nsteps : nullptr, MCD_MEM_HOST,
+                                           &st2, false, &bad_b);
+    if (rc2 != MCD_OK && rc2 != MCD_ERR_NOT_CONVERGED) return rc2;
+    g = st2.cert_rel_gap;
+    if (stats) stats->sweep_fallbacks += 1;
+    return MCD_OK;
+  };
+  return sweep_replicates(h, P, nrep, m_sub, n_sub, assign, step, step_obj, cert_gap, stats, hk);
+}
+
+// Placement of the left-out cells of the replicates [r0, r0 + nb) (blocks at `out`, layout L) and the copies of
+// their results into the dense host outputs.
+static int loo_place_batch(mcd_context* h, const int* d_cells, int64_t r0, int64_t nb, int64_t m_sub, int64_t nsteps,
+                           int64_t k_steps, char* out, const mcd_loo_layout& L, int32_t* test_col, double* test_corr,
+                           double* total, double* match_corr) {
+  int st;
+  if ((st = mcd_launch_loo_place(h, static_cast<const double*>(h->ws[WS_C].ptr), h->last_ldc, d_cells + r0, nb, m_sub,
+                                 h->last_N, nsteps, k_steps, out, L)))
+    return st;
+  MCD_CUDA(h, cudaMemcpy2DAsync(test_corr + r0, 8, out + L.res, L.stride, 8, (size_t)nb, cudaMemcpyDeviceToHost, h->stream));
+  MCD_CUDA(h, cudaMemcpy2DAsync(total + r0, 8, out + L.res + 8, L.stride, 8, (size_t)nb, cudaMemcpyDeviceToHost, h->stream));
+  MCD_CUDA(h, cudaMemcpy2DAsync(test_col + r0, 4, out + L.res + 16, L.stride, 4, (size_t)nb, cudaMemcpyDeviceToHost,
+                                h->stream));
+  if (match_corr && m_sub > 0)
+    MCD_CUDA(h, cudaMemcpy2DAsync(match_corr + r0 * m_sub, (size_t)m_sub * 8, out + L.match, L.stride, (size_t)m_sub * 8,
+                                  (size_t)nb, cudaMemcpyDeviceToHost, h->stream));
+  return MCD_OK;
+}
+
+int mcd_loo_sweep(mcd_handle h, const int32_t* cells, int64_t ncells, int64_t k_steps, int32_t* test_col,
+                  double* test_corr, double* total, int32_t* assign, int32_t* step, double* step_obj, double* match_corr,
+                  double* cert_gap, int concurrency, mcd_stats* stats) {
+  if (!h) return MCD_ERR_INVALID;
+  if (h->last_M < 1 || h->last_assign == nullptr)
+    return mcd_fail(h, MCD_ERR_INVALID, "mcd_loo_sweep: no mcd_cell2cell result is resident");
+  if (!cells || ncells < 1) return mcd_fail(h, MCD_ERR_INVALID, "mcd_loo_sweep: no cells to leave out");
+  if (k_steps < 1) return mcd_fail(h, MCD_ERR_INVALID, "mcd_loo_sweep: k_steps must be >= 1");
+  if (!test_col || !test_corr || !total)
+    return mcd_fail(h, MCD_ERR_INVALID, "mcd_loo_sweep: test_col, test_corr and total are required");
+  for (int64_t r = 0; r < ncells; ++r)
+    if (cells[r] < 0 || cells[r] >= h->last_M) return mcd_fail(h, MCD_ERR_INVALID, "mcd_loo_sweep: cell out of range");
+  MCD_CUDA(h, cudaSetDevice(h->device));
+  const int64_t N = h->last_N, m_sub = h->last_M - 1;
+  const double* C = static_cast<const double*>(h->ws[WS_C].ptr);
+  const int64_t ldc = h->last_ldc;
+  int st;
+  void* p_idx = nullptr;
+  if ((st = mcd_ws(h, WS_SWEEP_IDX, (size_t)ncells * 4, &p_idx))) return st;
+  const int* d_cells = static_cast<const int*>(p_idx);
+  MCD_CUDA(h, cudaMemcpyAsync(p_idx, cells, (size_t)ncells * 4, cudaMemcpyHostToDevice, h->stream));
+  // the replicate's extra bytes after its StepOut block: match counts [N], results, matched correlations [m_sub]
+  const size_t cnt_bytes = ((size_t)N * 4 + 255) / 256 * 256, res_bytes = 256;
+  const size_t mc_bytes = match_corr ? ((size_t)m_sub * 8 + 255) / 256 * 256 : 0;
+  mcd_loo_layout L;
+  if (m_sub == 0) {
+    // M == 1: every replicate is empty, no solve runs; the placement sees no matches at all
+    L.stride = cnt_bytes + res_bytes;
+    L.assign = L.obj = L.cnt = 0;
+    L.res = cnt_bytes;
+    L.match = 0;
+    void* p_out = nullptr;
+    if ((st = mcd_ws(h, WS_SWEEP_OUT, (size_t)ncells * L.stride, &p_out))) return st;
+    const int64_t launches0 = h->launches;
+    MCD_CUDA(h, cudaEventRecord(get_event(h, 96), h->stream));
+    if ((st = loo_place_batch(h, d_cells, 0, ncells, 0, 0, k_steps, static_cast<char*>(p_out), L, test_col, test_corr,
+                              total, nullptr)))
+      return st;
+    MCD_CUDA(h, cudaEventRecord(get_event(h, 97), h->stream));
+    MCD_CUDA(h, cudaStreamSynchronize(h->stream));
+    for (int64_t r = 0; cert_gap && r < ncells; ++r) cert_gap[r] = h->opt.certify ? 0.0 : -1.0;
+    if (stats) {
+      memset(stats, 0, sizeof *stats);
+      float ms = 0.f;
+      cudaEventElapsedTime(&ms, get_event(h, 96), get_event(h, 97));
+      stats->ms_lap = ms;
+      stats->ms_total = ms;
+      stats->kernel_launches = h->launches - launches0;
+    }
+    return MCD_OK;
+  }
+  const SweepPlan P = sweep_plan(ncells, m_sub, N, cnt_bytes + res_bytes + mc_bytes, concurrency);
+  L.stride = P.rep_bytes;
+  L.cnt = P.step_bytes;
+  L.res = P.step_bytes + cnt_bytes;
+  L.match = match_corr ? P.step_bytes + cnt_bytes + res_bytes : 0;
+  SweepHooks hk;
+  hk.build = [&](mcd_context* w, int64_t r0, int64_t b, double* subC, int64_t lds, double* subCt, int64_t ldst,
+                 const int** dna_class) -> int {
+    *dna_class = nullptr;  // no DNA cell is repeated: the asynchronous solver path
+    int stw = mcd_launch_loo_gather(w, C, ldc, cells[r0 + b], m_sub, N, subC, lds);
+    return stw ? stw : mcd_transpose_f64(w, subC, m_sub, N, lds, subCt, ldst);
+  };
+  hk.after = [&](int64_t r0, int64_t nb, char* out) -> int {
+    const StepOut o = carve_step_out(out, m_sub, P.nsteps);  // the step loop's outputs inside a replicate's block
+    L.assign = (size_t)(reinterpret_cast<char*>(o.assign) - out);
+    L.obj = (size_t)(reinterpret_cast<char*>(o.obj) - out);
+    return loo_place_batch(h, d_cells, r0, nb, m_sub, P.nsteps, k_steps, out, L, test_col, test_corr, total, match_corr);
+  };
+  return sweep_replicates(h, P, ncells, m_sub, N, assign, step, step_obj, cert_gap, stats, hk);
 }
 
 int mcd_null_assignments(mcd_handle h, int64_t trials, uint64_t seed, double* sums, double* medians, int out_space) {

@@ -164,6 +164,23 @@ int mcd_launch_corr_split(mcd_context* h, const uint16_t* A_hi, const uint16_t* 
 int mcd_launch_null_assignments(mcd_context* h, const double* C, int64_t ldc, int64_t M, int64_t N, int64_t trials,
                                 uint64_t seed, double* d_sums, double* d_medians);
 
+// Leave-one-out sweep (loo.cu).  Byte offsets inside one replicate's block of the sweep's output buffer.
+struct mcd_loo_layout {
+  size_t stride;  // bytes per replicate
+  size_t assign;  // int32 [m_sub]: DNA column of each remaining row (the replicate's step-loop output)
+  size_t obj;     // double [nsteps]: its step objectives
+  size_t cnt;     // int32 [N]: scratch, matches per DNA column
+  size_t res;     // double test_corr, double total, int32 test_col
+  size_t match;   // double [m_sub]: C[row, assign] of the remaining rows; 0 = not wanted
+};
+// sub [m, lds] = C [M, ldc] with row q deleted (rows in ascending order, columns [0, n))
+int mcd_launch_loo_gather(mcd_context* h, const double* C, int64_t ldc, int64_t q, int64_t m, int64_t n, double* sub,
+                          int64_t lds);
+// one CTA per replicate r < nrep (block at base + r * L.stride, left-out row d_cells[r]): placement of the left-out
+// cell, its correlation, the replicate's total and (L.match) the matched correlations
+int mcd_launch_loo_place(mcd_context* h, const double* C, int64_t ldc, const int* d_cells, int64_t nrep, int64_t m_sub,
+                         int64_t N, int64_t nsteps, int64_t k_steps, char* base, const mcd_loo_layout& L);
+
 struct mcd_lap_counters {  // device-resident, one per solve
   long long rounds;
   long long bids;
