@@ -316,7 +316,23 @@ int mcd_corr_pairs(mcd_handle h, const int32_t* rows, const int32_t* cols, int64
  * Random-assignment null test on the resident correlation matrix (random_assignment_test.py:233-258,
  * random_assignment_test_median.py): `trials` independent random step-wise injective assignments; sums [trials]
  * = sum of the matched correlations, medians [trials] = their median (NULL to skip).  Same distribution as the
- * reference's np.random.choice chain, not the same random stream.  At most 4096 cells per side.
+ * reference's np.random.choice chain, not the same random stream.
+ *
+ * The draw of trial t (0 <= t < trials) of `seed` on the resident M x N matrix C, with mix64 the splitmix64
+ * finaliser and all arithmetic in wrapping uint64:
+ *   base = mix64(seed ^ mix64(t));  b = max(13, bit_length(max(M, N) - 1)) index bits;
+ *   RNA key of row i    = ((mix64(base + 2i)     >> b) << b) | i,
+ *   DNA key of column j = ((mix64(base + 2j + 1) >> b) << b) | j;
+ *   q, r = divmod(M, N).  The RNA rows are taken in ascending key order; position p < q N takes DNA column p mod N,
+ *   position p >= q N the DNA column with the (p - q N)-th smallest DNA key.
+ *   sums[t] = the FP64 sum of the M matched values C[row, col]; medians[t] = 0.5 (v[(M-1)/2] + v[M/2]) of the sorted
+ *   values (numpy.median).
+ * A trial depends only on (seed, t, C): not on `trials`, the launch or the kernel that computes it.  The one
+ * deviation from a uniformly random permutation: two keys with equal hash bits are ordered by index; the chance of
+ * such a tie in a trial is about M^2 / 2^(65-b) (4e-6 at 50 000 x 10 000).  More than 2^24 cells on a side (fewer
+ * than 40 hash bits) returns MCD_ERR_UNSUPPORTED.  Up to 4096 cells a side the keys are sorted in shared memory;
+ * above, in per-CTA global scratch of its own (<= 1 GiB), so the resident matrix and the last run's outputs are
+ * untouched.  Measured throughput: DESIGN.md section 4, "Views of the resident matrix".
  */
 int mcd_null_assignments(mcd_handle h, int64_t trials, uint64_t seed, double* sums, double* medians, int out_space);
 

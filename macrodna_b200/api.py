@@ -477,7 +477,8 @@ class random_test:
     The matrix is computed once on the device (the constructor runs the hot path); ``assign()`` returns the sum of
     the matched correlations of ONE random assignment like the reference, drawn from batches generated by
     ``mcd_null_assignments``; ``assign_many`` returns a whole batch (optionally with the medians of
-    random_assignment_test_median.py).  Same distribution as the reference, not NumPy's random stream."""
+    random_assignment_test_median.py).  Same distribution as the reference, not NumPy's random stream; every trial is
+    the draw written down at ``mcd_null_assignments`` (include/macrodna_b200.h), up to 2^24 cells a side."""
 
     def __init__(self, rna_df=None, dna_df=None, *, device=0, precision="ozaki", seed=2023, batch=4096):
         self._m = MaCroDNA(rna_df, dna_df, device=device, precision=precision)

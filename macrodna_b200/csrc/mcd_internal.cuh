@@ -108,6 +108,7 @@ enum {
   WS_SUB_MISC,
   WS_SWEEP_IDX,  // replicate sweep: RNA rows + the batch's DNA columns
   WS_SWEEP_OUT,  // replicate sweep: per-replicate step-loop outputs of the batch
+  WS_NULL,       // null test above 4096 cells a side: per-CTA key slabs (<= 1 GiB)
 };
 
 int mcd_fail(mcd_context* h, int status, const char* what, cudaError_t e = cudaSuccess);
