@@ -107,7 +107,7 @@ void* mcd_stream(mcd_handle h);
  * as -1), "deterministic" (0; 1 = round-synchronous solver kernels only: the bid order, and with it the optimum
  * picked on inputs with exact ties, is then fixed; the default asynchronous kernel of the rectangular steps gives the
  * same unique optimum on tie-free inputs and redoes a step synchronously when it meets exact ties), "ozaki.slices" (0 = auto),
- * "ozaki.align", "ozaki.plan", "k1.generic", "k1.no_stream", and the solver knobs "lap.theta", "lap.eps_min", "lap.eps0", "lap.scaling",
+ * "ozaki.radix" (0 = auto; 128 or 256 forces the digit radix, see mcd_ozaki_format), "ozaki.align", "ozaki.plan", "k1.generic", "k1.no_stream", and the solver knobs "lap.theta", "lap.eps_min", "lap.eps0", "lap.scaling",
  * "lap.max_rounds", "lap.tail_budget", "lap.blocks_per_sm", "lap.grid_blocks", "lap.list_max_m", "lap.lists", "lap.list_min_nu",
  * "lap.tail_cluster", "lap.tail_mh", "lap.tail_sym", "lap.async", "lap.async_nu", "lap.async_threads", "lap.async_blocks_per_sm", "lap.async_stop", "lap.prefetch_rows", "lap.tail_nu", "lap.mh_nu", "lap.scale_cut", "lap.scale_tail_rounds", "lap.scale_full_phases", "lap.aug_nu", "lap.aug_nu_square", "lap.rank_select",
  * "lap.min_chunk", "lap.chunk_waves".  Unknown names return MCD_ERR_INVALID.
@@ -139,13 +139,25 @@ int mcd_standardize_split(mcd_handle h, const double* X, int64_t ncells, int64_t
  *   digits [nsl, ncells, ldk8] int8, ldk8 = mcd_padded_k_split(G), zero padded;  scale [ncells] = 2^-e (the
  *   factor that undoes the row scaling);  nsl in [2, 8] (mcd_ozaki_default_slices(): 6). */
 int mcd_ozaki_default_slices(void);
-/* Slice count the fused driver uses for an M x N x G instance: 8 (FP64-GEMM-level error) while M*N*G <= 2e11,
- * 6 (~1e-12 absolute) above; the handle option "ozaki.slices" overrides. */
+/* Digit format the drivers use for an M x N x G instance on handle h (NULL: no handle options), ldk8 =
+ * mcd_padded_k_split(G):
+ *   "ozaki.slices" set: that many radix-128 slices (radix 256 if "ozaki.radix" is 256 too; at most 7 slices then);
+ *   else "ozaki.radix" 256: 5 radix-256 slices;  else M*N*G <= 2e11 (or "ozaki.radix" 128): 8 radix-128 slices
+ *   (FP64-GEMM-level error), 6 above M*N*G > 2e11;
+ *   else ldk8 <= 32 704: 5 radix-256 slices (15 products, ~5e-12 absolute);  else 6 radix-128 slices (21 products).
+ * Writes *nsl and *radix_bits (7 = radix 128, 8 = radix 256).  Returns 1 if the int32 accumulators of
+ * mcd_corr_ozaki_radix are exact at this ldk8 in that format, 0 if the drivers take the FP64 pipe instead. */
+int mcd_ozaki_format(mcd_handle h, int64_t M, int64_t N, int64_t G, int* nsl, int* radix_bits);
+/* The slice count of mcd_ozaki_format without handle options (5 at radix-256 shapes). */
 int mcd_ozaki_slices_for(int64_t M, int64_t N, int64_t G);
-/* The slice count a given handle will use: its "ozaki.slices" option if set, else mcd_ozaki_slices_for. */
+/* The slice count of mcd_ozaki_format for a given handle. */
 int mcd_ozaki_slices(mcd_handle h, int64_t M, int64_t N, int64_t G);
 int mcd_standardize_ozaki(mcd_handle h, const double* X, int64_t ncells, int64_t G, int64_t ldx, int8_t* digits,
                           int nsl, double* scale, double* norms);
+/* Same with digits of radix_bits bits: 7 = the radix-128 digits above; 8 = balanced radix-256 digits in
+ * [-128, 127] of rint(u * 2^(8 nsl - 1)) (the leading one in [-64, 64]), nsl in [2, 7]. */
+int mcd_standardize_ozaki_radix(mcd_handle h, const double* X, int64_t ncells, int64_t G, int64_t ldx, int8_t* digits,
+                                int nsl, int radix_bits, double* scale, double* norms);
 /* Synchronise and return MCD_ERR_NONFINITE if any standardise call since the last check saw NaN/Inf. */
 int mcd_check_finite(mcd_handle h);
 
@@ -170,6 +182,11 @@ int mcd_corr_split(mcd_handle h, const uint16_t* A3, int64_t M, const uint16_t* 
 int mcd_corr_ozaki(mcd_handle h, const int8_t* A8, int64_t M, const int8_t* B8, int64_t N, int64_t G, int64_t ldk8,
                    int nsl, const double* sA, const double* sB, const double* nA, const double* nB, double* C,
                    int64_t ldc, double* Ct, int64_t ldct);
+/* Same on the digits of mcd_standardize_ozaki_radix.  radix_bits 8: MCD_ERR_UNSUPPORTED if
+ * 16384 (nsl - 1) ldk8 >= 2^31 (5 slices: ldk8 <= 32 704). */
+int mcd_corr_ozaki_radix(mcd_handle h, const int8_t* A8, int64_t M, const int8_t* B8, int64_t N, int64_t G,
+                         int64_t ldk8, int nsl, int radix_bits, const double* sA, const double* sB, const double* nA,
+                         const double* nB, double* C, int64_t ldc, double* Ct, int64_t ldct);
 
 /*
  * K3 -- one rectangular assignment.  Replaces one `ilp` call (macrodna.py:27-84):

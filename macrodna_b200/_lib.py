@@ -87,8 +87,12 @@ SIGNATURES = {
     "mcd_ozaki_default_slices": (_I, []),
     "mcd_ozaki_slices_for": (_I, [_I64, _I64, _I64]),
     "mcd_ozaki_slices": (_I, [_VP, _I64, _I64, _I64]),
+    "mcd_ozaki_format": (_I, [_VP, _I64, _I64, _I64, C.POINTER(_I), C.POINTER(_I)]),
     "mcd_standardize_ozaki": (_I, [_VP, _VP, _I64, _I64, _I64, _VP, _I, _VP, _VP]),
+    "mcd_standardize_ozaki_radix": (_I, [_VP, _VP, _I64, _I64, _I64, _VP, _I, _I, _VP, _VP]),
     "mcd_corr_ozaki": (_I, [_VP, _VP, _I64, _VP, _I64, _I64, _I64, _I, _VP, _VP, _VP, _VP, _VP, _I64, _VP, _I64]),
+    "mcd_corr_ozaki_radix": (_I, [_VP, _VP, _I64, _VP, _I64, _I64, _I64, _I, _I, _VP, _VP, _VP, _VP, _VP, _I64, _VP,
+                                  _I64]),
     "mcd_check_finite": (_I, [_VP]),
     "mcd_corr_fp64": (_I, [_VP, _VP, _I64, _VP, _I64, _I64, _I64, _VP, _VP, _VP, _I64, _VP, _I64]),
     "mcd_corr_split": (_I, [_VP, _VP, _I64, _VP, _I64, _I64, _I64, _VP, _VP, _VP, _I64, _VP, _I64]),
@@ -249,6 +253,13 @@ class Handle:
         v = C.c_double()
         self.check(self.lib.mcd_get_option(self.h, name.encode(), C.byref(v)))
         return v.value
+
+    def ozaki_format(self, M, N, G):
+        """(nsl, radix_bits, exact) of ``mcd_ozaki_format``: the digit format this handle uses for M x N x G, and
+        whether its int32 accumulation is exact there (False: the drivers take the FP64 pipe)."""
+        nsl, rb = C.c_int(), C.c_int()
+        exact = self.lib.mcd_ozaki_format(self.h, M, N, G, C.byref(nsl), C.byref(rb))
+        return nsl.value, rb.value, exact == 1
 
     @property
     def sm_count(self):

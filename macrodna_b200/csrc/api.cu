@@ -151,16 +151,44 @@ int mcd_standardize_split(mcd_handle h, const double* X, int64_t ncells, int64_t
 
 int mcd_ozaki_default_slices(void) { return 6; }
 
+int mcd_ozaki_format(mcd_handle h, int64_t M, int64_t N, int64_t G, int* nsl, int* radix_bits) {
+  if (!nsl || !radix_bits) return MCD_ERR_INVALID;
+  const int64_t ldk8 = mcd_padded_k_split(G);
+  const int slices = h != nullptr ? h->opt.ozaki_slices : 0;
+  const int radix = h != nullptr ? h->opt.ozaki_radix : 0;  // 128 / 256 forced, anything else automatic
+  const bool cheap = (double)M * (double)N * (double)G <= 2.0e11;
+  int n, rb;
+  if (slices >= 2) {
+    // an explicit slice count keeps radix 128 unless the radix is forced too (radix 256 carries at most 7 slices)
+    rb = radix == 256 ? 8 : 7;
+    n = slices > (rb == 8 ? 7 : MCD_OZAKI_MAX_SLICES) ? (rb == 8 ? 7 : MCD_OZAKI_MAX_SLICES) : slices;
+  } else if (radix == 256) {
+    rb = 8, n = 5;
+  } else if (cheap || radix == 128) {
+    // 8 slices (36 products, error at the level of an FP64 GEMM's own rounding) while the contraction is cheap
+    // anyway; 6 slices (21 products, ~1e-12 absolute) above
+    rb = 7, n = cheap ? 8 : 6;
+  } else if (mcd_ozaki_exact(5, 8, ldk8)) {
+    // the large-instance bottleneck: 5 radix-256 slices (15 products, ~5e-12 absolute) up to ldk8 = 32 704
+    rb = 8, n = 5;
+  } else {
+    rb = 7, n = 6;
+  }
+  *nsl = n;
+  *radix_bits = rb;
+  return mcd_ozaki_exact(n, rb, ldk8) ? 1 : 0;
+}
+
 int mcd_ozaki_slices_for(int64_t M, int64_t N, int64_t G) {
-  // 8 slices (36 products, error at the level of an FP64 GEMM's own rounding) while the contraction is cheap
-  // anyway; 6 slices (21 products, ~1e-12 absolute) once it is the large-instance bottleneck
-  return (double)M * (double)N * (double)G <= 2.0e11 ? 8 : 6;
+  int nsl = 0, rb = 0;
+  mcd_ozaki_format(nullptr, M, N, G, &nsl, &rb);
+  return nsl;
 }
 
 int mcd_ozaki_slices(mcd_handle h, int64_t M, int64_t N, int64_t G) {
-  if (h != nullptr && h->opt.ozaki_slices >= 2)
-    return h->opt.ozaki_slices > MCD_OZAKI_MAX_SLICES ? MCD_OZAKI_MAX_SLICES : h->opt.ozaki_slices;
-  return mcd_ozaki_slices_for(M, N, G);
+  int nsl = 0, rb = 0;
+  mcd_ozaki_format(h, M, N, G, &nsl, &rb);
+  return nsl;
 }
 
 namespace {
@@ -177,6 +205,7 @@ const OptEntry kOptions[] = {
     MCD_OPT_I("corr_only", corr_only),
     MCD_OPT_I("deterministic", deterministic),
     MCD_OPT_I("ozaki.slices", ozaki_slices),
+    MCD_OPT_I("ozaki.radix", ozaki_radix),
     MCD_OPT_I("ozaki.align", ozaki_align),
     MCD_OPT_I("ozaki.plan", ozaki_plan),
     MCD_OPT_I("k1.generic", k1_generic),
@@ -242,11 +271,11 @@ int mcd_get_option(mcd_handle h, const char* name, double* value) {
   return MCD_OK;
 }
 
-int mcd_standardize_ozaki(mcd_handle h, const double* X, int64_t ncells, int64_t G, int64_t ldx, int8_t* digits,
-                          int nsl, double* scale, double* norms) {
+int mcd_standardize_ozaki_radix(mcd_handle h, const double* X, int64_t ncells, int64_t G, int64_t ldx, int8_t* digits,
+                                int nsl, int radix_bits, double* scale, double* norms) {
   if (!h) return MCD_ERR_INVALID;
   if (!X || !digits || !scale || !norms || ncells < 0 || G < 1 || ldx < G || G > 0x7fffffff || nsl < 2 ||
-      nsl > MCD_OZAKI_MAX_SLICES)
+      (radix_bits != 7 && radix_bits != 8) || nsl > (radix_bits == 8 ? 7 : MCD_OZAKI_MAX_SLICES))
     return mcd_fail(h, MCD_ERR_INVALID, "mcd_standardize_ozaki arguments");
   MCD_CUDA(h, cudaSetDevice(h->device));
   mcd_ozaki_out oz;
@@ -254,19 +283,32 @@ int mcd_standardize_ozaki(mcd_handle h, const double* X, int64_t ncells, int64_t
   oz.ldk8 = mcd_padded_k_split(G);
   oz.slice_stride = ncells * oz.ldk8;
   oz.nsl = nsl;
+  oz.rb = radix_bits;
   oz.scale = scale;
   return mcd_launch_standardize(h, X, ncells, G, ldx, nullptr, 0, nullptr, nullptr, 0, norms, nullptr, &oz);
 }
 
-int mcd_corr_ozaki(mcd_handle h, const int8_t* A8, int64_t M, const int8_t* B8, int64_t N, int64_t G, int64_t ldk8,
-                   int nsl, const double* sA, const double* sB, const double* nA, const double* nB, double* C,
-                   int64_t ldc, double* Ct, int64_t ldct) {
+int mcd_standardize_ozaki(mcd_handle h, const double* X, int64_t ncells, int64_t G, int64_t ldx, int8_t* digits,
+                          int nsl, double* scale, double* norms) {
+  return mcd_standardize_ozaki_radix(h, X, ncells, G, ldx, digits, nsl, 7, scale, norms);
+}
+
+int mcd_corr_ozaki_radix(mcd_handle h, const int8_t* A8, int64_t M, const int8_t* B8, int64_t N, int64_t G,
+                         int64_t ldk8, int nsl, int radix_bits, const double* sA, const double* sB, const double* nA,
+                         const double* nB, double* C, int64_t ldc, double* Ct, int64_t ldct) {
   if (!h) return MCD_ERR_INVALID;
   if (!A8 || !B8 || !sA || !sB || !nA || !nB || (!C && !Ct) || M < 0 || N < 0 || G < 1 || ldk8 < G ||
       (ldk8 % 64) != 0 || (C && ldc < N) || (Ct && ldct < M))
     return mcd_fail(h, MCD_ERR_INVALID, "mcd_corr_ozaki arguments");
   MCD_CUDA(h, cudaSetDevice(h->device));
-  return mcd_launch_corr_ozaki(h, A8, M * ldk8, M, B8, N * ldk8, N, ldk8, nsl, sA, sB, nA, nB, C, ldc, Ct, ldct);
+  return mcd_launch_corr_ozaki(h, A8, M * ldk8, M, B8, N * ldk8, N, ldk8, nsl, radix_bits, sA, sB, nA, nB, C, ldc, Ct,
+                               ldct);
+}
+
+int mcd_corr_ozaki(mcd_handle h, const int8_t* A8, int64_t M, const int8_t* B8, int64_t N, int64_t G, int64_t ldk8,
+                   int nsl, const double* sA, const double* sB, const double* nA, const double* nB, double* C,
+                   int64_t ldc, double* Ct, int64_t ldct) {
+  return mcd_corr_ozaki_radix(h, A8, M, B8, N, G, ldk8, nsl, 7, sA, sB, nA, nB, C, ldc, Ct, ldct);
 }
 
 int mcd_check_finite(mcd_handle h) {
@@ -849,10 +891,9 @@ int mcd_cell2cell_gather(mcd_handle h, const double* rna, int64_t ld_rna, const 
   }
   if (precision != MCD_PREC_FP64 && precision != MCD_PREC_SPLIT_FP16 && precision != MCD_PREC_OZAKI_INT8)
     return mcd_fail(h, MCD_ERR_INVALID, "unknown precision");
-  const int nsl = mcd_ozaki_slices(h, M, N, G);
+  int nsl = 0, rb = 0;
   // exact int32 accumulation bounds the gene count of the integer path; longer rows use the FP64 pipe
-  if (precision == MCD_PREC_OZAKI_INT8 && (double)nsl * 4096.0 * (double)mcd_padded_k_split(G) >= 2147483648.0)
-    precision = MCD_PREC_FP64;
+  if (mcd_ozaki_format(h, M, N, G, &nsl, &rb) != 1 && precision == MCD_PREC_OZAKI_INT8) precision = MCD_PREC_FP64;
   MCD_CUDA(h, cudaSetDevice(h->device));
   h->last_M = 0;  // whatever was resident is about to be overwritten (also on an early error return)
   h->last_assign = nullptr;
@@ -947,6 +988,7 @@ int mcd_cell2cell_gather(mcd_handle h, const double* rna, int64_t ld_rna, const 
   ozb.ldk8 = ldk;
   ozb.slice_stride = N * ldk;
   ozb.nsl = nsl;
+  ozb.rb = rb;
   ozb.scale = sB;
   oza = ozb;
   oza.slice_stride = M * ldk;
@@ -993,7 +1035,7 @@ int mcd_cell2cell_gather(mcd_handle h, const double* rna, int64_t ld_rna, const 
       if ((st = mcd_launch_standardize(h, xr, mr, G, ldr, nullptr, 0, nullptr, nullptr, 0, nA + r0, d_ridx, &oza)))
         return st;
       MCD_CUDA(h, cudaEventRecord(get_event(h, EV_CHUNK + 4 * c + 2), h->stream));
-      if ((st = mcd_launch_corr_ozaki(h, oza.digits, oza.slice_stride, mr, ozb.digits, ozb.slice_stride, N, ldk, nsl,
+      if ((st = mcd_launch_corr_ozaki(h, oza.digits, oza.slice_stride, mr, ozb.digits, ozb.slice_stride, N, ldk, nsl, rb,
                                       sA + r0, sB, nA + r0, nB, C + r0 * ldc, ldc, Ct + r0, ldct)))
         return st;
     } else {
@@ -1095,7 +1137,7 @@ struct ShardOperands {
 // K1 of both operands + K2 of `rows` RNA rows on handle h; C_loc [rows, ldc] (no transpose).  All on h->stream.
 int shard_standardize_correlate(mcd_context* h, const double* d_rna, int64_t ldr, const int* d_ridx, const double* d_dna,
                                 int64_t ldd, const int* d_didx, int64_t rows, int64_t N, int64_t G, int precision, int nsl,
-                                double* C_loc, int64_t ldc) {
+                                int rb, double* C_loc, int64_t ldc) {
   int st;
   ShardOperands o;
   void *pnA = nullptr, *pnB = nullptr;
@@ -1125,6 +1167,7 @@ int shard_standardize_correlate(mcd_context* h, const double* d_rna, int64_t ldr
     ozb.ldk8 = ldk;
     ozb.slice_stride = N * ldk;
     ozb.nsl = nsl;
+    ozb.rb = rb;
     ozb.scale = o.sB;
     oza = ozb;
     oza.digits = static_cast<int8_t*>(o.pa);
@@ -1133,7 +1176,7 @@ int shard_standardize_correlate(mcd_context* h, const double* d_rna, int64_t ldr
     if ((st = mcd_launch_standardize(h, d_dna, N, G, ldd, nullptr, 0, nullptr, nullptr, 0, o.nB, d_didx, &ozb))) return st;
     if (rows > 0) {
       if ((st = mcd_launch_standardize(h, d_rna, rows, G, ldr, nullptr, 0, nullptr, nullptr, 0, o.nA, d_ridx, &oza))) return st;
-      st = mcd_launch_corr_ozaki(h, oza.digits, oza.slice_stride, rows, ozb.digits, ozb.slice_stride, N, ldk, nsl, o.sA, o.sB,
+      st = mcd_launch_corr_ozaki(h, oza.digits, oza.slice_stride, rows, ozb.digits, ozb.slice_stride, N, ldk, nsl, rb, o.sA, o.sB,
                                  o.nA, o.nB, C_loc, ldc, nullptr, 0);
     }
   } else {
@@ -1170,9 +1213,8 @@ int mcd_cell2cell_multi(mcd_handle* hs, int ndev, const double* rna, int64_t ld_
     if ((rna_gene_idx && (rna_gene_idx[g] < 0 || rna_gene_idx[g] >= ld_rna)) ||
         (dna_gene_idx && (dna_gene_idx[g] < 0 || dna_gene_idx[g] >= ld_dna)))
       return mcd_fail(h0, MCD_ERR_INVALID, "mcd_cell2cell_multi: gene index out of range");
-  const int nsl = mcd_ozaki_slices(h0, M, N, G);
-  if (precision == MCD_PREC_OZAKI_INT8 && (double)nsl * 4096.0 * (double)mcd_padded_k_split(G) >= 2147483648.0)
-    precision = MCD_PREC_FP64;
+  int nsl = 0, rb = 0;
+  if (mcd_ozaki_format(h0, M, N, G, &nsl, &rb) != 1 && precision == MCD_PREC_OZAKI_INT8) precision = MCD_PREC_FP64;
   h0->last_M = 0;
   h0->last_assign = nullptr;
   const int64_t ldc = (N + 1) & ~1LL, ldct = (M + 1) & ~1LL;
@@ -1231,7 +1273,7 @@ int mcd_cell2cell_multi(mcd_handle* hs, int ndev, const double* rna, int64_t ld_
       MCD_CUDA(h0, cudaStreamWaitEvent(h->stream, get_event(h0, 0), 0));
     }
     if ((st = shard_standardize_correlate(h, static_cast<const double*>(pr), wr, d_ridx, static_cast<const double*>(pd), wd,
-                                          d_didx, rows, N, G, precision, nsl, C_loc, ldc)))
+                                          d_didx, rows, N, G, precision, nsl, rb, C_loc, ldc)))
       return mcd_fail(h0, st, h->err.c_str());
     if (d > 0 && rows > 0)
       MCD_CUDA(h0, cudaMemcpyPeerAsync(C + lo * ldc, h0->device, C_loc, h->device, (size_t)rows * ldc * 8, h->stream));

@@ -2,15 +2,16 @@
 //
 // Replaces the RNA x DNA double loop of the reference (src/MaCroDNA/macrodna.py:103-107) with an
 // error-free ("Ozaki scheme") integer GEMM.  K1 writes every unit-norm centred row as nsl balanced
-// radix-128 digit slices (int8, standardize.cu::ozaki_digits):
-//     x = 2^-(7 nsl - 1) * sum_t d_t 128^(nsl-1-t),   d_t in [-64, 63].
+// digit slices of rb bits (int8, standardize.cu::ozaki_digits / ozaki_digits256):
+//     x = 2^-(rb nsl - 1) * sum_t d_t 2^(rb (nsl-1-t)),   d_t in [-64, 63] (rb = 7) or [-128, 127] (rb = 8).
 // A dot product then splits into digit-slice products that the tensor core evaluates EXACTLY
 // (int8 x int8 -> int32, no rounding anywhere):
-//     <x, y> = 2^-12 * sum_g 2^(-7 g) ACC_g,    ACC_g = sum_{t+t'=g} sum_k d_t[k] d'_t'[k],
+//     <x, y> = 2^(2 - 2 rb) * sum_g 2^(-rb g) ACC_g,    ACC_g = sum_{t+t'=g} sum_k d_t[k] d'_t'[k],
 // truncated at g < nsl (the dropped groups are below the digit resolution).  All products of one
-// significance group g share ONE int32 accumulator in TMEM (|ACC_g| <= (g+1) * 4096 * K < 2^31), the FP64
-// combination of the groups happens once per output in the epilogue.  nsl = 6 (21 products) gives
-// ~1e-12 absolute, nsl = 8 (36 products) is at the level of an FP64 GEMM's own rounding.
+// significance group g share ONE int32 accumulator in TMEM (the caller keeps |ACC_g| < 2^31:
+// mcd_ozaki_exact), the FP64 combination of the groups happens once per output in the epilogue.
+// Radix 128: nsl = 6 (21 products) gives ~1e-12 absolute, nsl = 8 (36 products) is at the level of an FP64
+// GEMM's own rounding.  Radix 256: nsl = 5 (15 products) carries 40 bits, ~5e-12 absolute.
 //
 // Structure: persistent kernel, CTA PAIRS (cluster of 2, tcgen05 cta_group::2) on 256 x 256 output tiles:
 //   * each CTA stages 128 rows of the RNA tile and 128 rows of the DNA tile per digit slice (8 KB tiles,
@@ -398,6 +399,7 @@ struct OzParams {
   int64_t M, N;
   int num_kb;
   int nsl;
+  int rb;  // radix bits of the digits (7 or 8)
   int tiles_m, tiles_n;
   const double* sA;
   const double* sB;
@@ -551,7 +553,8 @@ corr_ozaki_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
         const int g_lo = 2 * ps;
         const bool two = p.nsl - g_lo >= 2;
         const bool first = ps == npass - 1, last = ps == 0;
-        const double w0 = scalbn(1.0, -7 * g_lo), w1 = scalbn(1.0, -7 * (g_lo + 1));
+        const double w0 = scalbn(1.0, -p.rb * g_lo), w1 = scalbn(1.0, -p.rb * (g_lo + 1));
+        const double fin = scalbn(1.0, 2 - 2 * p.rb);
         mbar_wait(tfull_bar, tphase);
         tphase ^= 1;
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
@@ -586,8 +589,8 @@ corr_ozaki_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
                 if (last) {
                   const int64_t col = col0 + 2 * q2;
                   const double nn0 = na * __ldg(p.nB + col), nn1 = na * __ldg(p.nB + col + 1);
-                  v0 = v0 * (sa * __ldg(p.sB + col) * (1.0 / 4096.0)) * (nn0 / (1e-10 + nn0));
-                  v1 = v1 * (sa * __ldg(p.sB + col + 1) * (1.0 / 4096.0)) * (nn1 / (1e-10 + nn1));
+                  v0 = v0 * (sa * __ldg(p.sB + col) * fin) * (nn0 / (1e-10 + nn0));
+                  v1 = v1 * (sa * __ldg(p.sB + col + 1) * fin) * (nn1 / (1e-10 + nn1));
                   if (p.Ct) {
                     p.Ct[col * p.ldct + row] = v0;
                     p.Ct[(col + 1) * p.ldct + row] = v1;
@@ -607,7 +610,7 @@ corr_ozaki_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_consta
                 if (last) {
                   const double nn = na * __ldg(p.nB + col);
                   // <u_i, u_j> * nn/(1e-10+nn) == dot(xc, yc)/(1e-10 + |xc||yc|)  (macrodna.py:25)
-                  v = v * (sa * __ldg(p.sB + col) * (1.0 / 4096.0)) * (nn / (1e-10 + nn));
+                  v = v * (sa * __ldg(p.sB + col) * fin) * (nn / (1e-10 + nn));
                   if (p.C) p.C[row * p.ldc + col] = v;
                   if (p.Ct) p.Ct[col * p.ldct + row] = v;
                 } else {
@@ -666,14 +669,14 @@ bool make_map(CUtensorMap* map, const int8_t* base, int64_t rows, int64_t ldk8, 
 }  // namespace
 
 int mcd_launch_corr_ozaki(mcd_context* h, const int8_t* A, int64_t a_stride, int64_t M, const int8_t* B,
-                          int64_t b_stride, int64_t N, int64_t ldk8, int nsl, const double* sA, const double* sB,
+                          int64_t b_stride, int64_t N, int64_t ldk8, int nsl, int rb, const double* sA, const double* sB,
                           const double* nA, const double* nB, double* C, int64_t ldc, double* Ct, int64_t ldct) {
   if (M == 0 || N == 0) return MCD_OK;
   if ((reinterpret_cast<uintptr_t>(A) & 15) || (reinterpret_cast<uintptr_t>(B) & 15) || (ldk8 % BK) != 0 ||
-      (a_stride & 15) || (b_stride & 15) || nsl < 2 || nsl > MCD_OZAKI_MAX_SLICES)
-    return mcd_fail(h, MCD_ERR_INVALID, "corr_ozaki: operands must be 16-byte aligned, ldk8 a multiple of 64, 2..8 slices");
-  // int32 accumulators: a group holds at most nsl products of |d d'| <= 4096 over ldk8 genes
-  if ((double)nsl * 4096.0 * (double)ldk8 >= 2147483648.0)
+      (a_stride & 15) || (b_stride & 15) || (rb != 7 && rb != 8) || nsl < 2 || nsl > (rb == 8 ? 7 : MCD_OZAKI_MAX_SLICES))
+    return mcd_fail(h, MCD_ERR_INVALID,
+                    "corr_ozaki: operands must be 16-byte aligned, ldk8 a multiple of 64, 2..8 slices of 7 bits or 2..7 of 8");
+  if (!mcd_ozaki_exact(nsl, rb, ldk8))
     return mcd_fail(h, MCD_ERR_UNSUPPORTED, "corr_ozaki: too many genes for exact int32 accumulation");
   CUtensorMap ma, mb;
   if (!make_map(&ma, A, M, ldk8, a_stride, nsl) || !make_map(&mb, B, N, ldk8, b_stride, nsl))
@@ -683,6 +686,7 @@ int mcd_launch_corr_ozaki(mcd_context* h, const int8_t* A, int64_t a_stride, int
   p.N = N;
   p.num_kb = (int)(ldk8 / BK);
   p.nsl = nsl;
+  p.rb = rb;
   p.tiles_m = (int)((M + TM - 1) / TM);
   p.tiles_n = (int)((N + TN - 1) / TN);
   p.sA = sA;

@@ -24,6 +24,7 @@ struct mcd_options {
   int corr_only = 0;          // "corr_only": mcd_cell2cell stops after K2 (matrix resident for the view calls)
   int deterministic = 0;      // "deterministic": round-synchronous solver kernels only (fixed bid order; see lap.async)
   int ozaki_slices = 0;       // "ozaki.slices": 0 = automatic (mcd_ozaki_slices_for)
+  int ozaki_radix = 0;        // "ozaki.radix": 128 or 256 forces the digit radix, 0 = automatic (mcd_ozaki_format)
   int ozaki_align = 1;        // "ozaki.align": wave alignment of the K2c producers
   int ozaki_plan = 1;         // "ozaki.plan": unit order of a K2c pass
   int k1_generic = 0;         // "k1.generic": force the generic digit kernel
@@ -136,14 +137,25 @@ int mcd_ws(mcd_context* h, int slot, size_t bytes, void** out);
 // int8 digit-slice operand of the Ozaki path (K1 output, K2c input):
 //   digits [nsl, ncells(+), ldk8] int8 -- slice t of row r starts at digits + t*slice_stride + r*ldk8
 //   scale  [ncells] double           -- 2^-e of the per-row power-of-two scaling
+//   rb     radix bits: 7 = balanced radix-128 digits in [-64, 63], 8 = balanced radix-256 digits in [-128, 127]
+//          (nsl <= 7: the fixed-point integer of 8 nsl - 1 bits must stay exact in a double's rounding)
 #define MCD_OZAKI_MAX_SLICES 8
 struct mcd_ozaki_out {
   int8_t* digits = nullptr;
   int64_t ldk8 = 0;
   int64_t slice_stride = 0;
   int nsl = 0;
+  int rb = 7;
   double* scale = nullptr;
 };
+// True if every significance-group sum of nsl slices over ldk8 genes is exact in K2c's int32 accumulators.
+// Radix 128: a group holds at most nsl products of |d d'| <= 4096.  Radix 256: the leading digit lies in [-64, 64]
+// (|q| <= 2^(8 nsl - 2)), the others in [-128, 127]; the heaviest group (g = nsl - 1) holds two products with the
+// leading digit (<= 64 * 128) and nsl - 2 others (<= 128 * 128): 16384 (nsl - 1) per gene.
+inline bool mcd_ozaki_exact(int nsl, int rb, int64_t ldk8) {
+  const double per_gene = rb == 8 ? 16384.0 * (nsl - 1) : 4096.0 * nsl;
+  return per_gene * (double)ldk8 < 2147483648.0;
+}
 
 // ---- kernel launchers (each returns an mcd_status) -------------------------------------------
 // slices_hi / slices_lo: the two fp16 slices (each [ncells, ldk16]); both NULL for the FP64 path
@@ -151,9 +163,9 @@ int mcd_launch_standardize(mcd_context* h, const double* X, int64_t ncells, int6
                            double* centred, int64_t ldk, uint16_t* slices_hi, uint16_t* slices_lo, int64_t ldk16,
                            double* norms, const int* gidx = nullptr, const mcd_ozaki_out* ozaki = nullptr);
 // K2c: C = sum over genes of the digit-slice products (exact int32 accumulation in TMEM), FP64 epilogue.
-// A: nsl slices of [M, ldk8] int8 (slice stride a_stride elements), B likewise; sA/sB the row scales.
+// A: nsl slices of [M, ldk8] int8 (slice stride a_stride elements), B likewise; sA/sB the row scales; rb radix bits.
 int mcd_launch_corr_ozaki(mcd_context* h, const int8_t* A, int64_t a_stride, int64_t M, const int8_t* B,
-                          int64_t b_stride, int64_t N, int64_t ldk8, int nsl, const double* sA, const double* sB,
+                          int64_t b_stride, int64_t N, int64_t ldk8, int nsl, int rb, const double* sA, const double* sB,
                           const double* nA, const double* nB, double* C, int64_t ldc, double* Ct, int64_t ldct);
 int mcd_launch_corr_fp64(mcd_context* h, const double* A, int64_t M, const double* B, int64_t N, int64_t ldk,
                          const double* nA, const double* nB, double* C, int64_t ldc, double* Ct, int64_t ldct);

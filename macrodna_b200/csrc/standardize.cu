@@ -85,6 +85,26 @@ __device__ __forceinline__ void ozaki_digits(double ys, int nsl, int d[MCD_OZAKI
     d[t] = (t < nsl) ? (int)((qb >> (7 * (nsl - 1 - t))) & 127ull) - 64 : 0;
 }
 
+// Radix-256 form (nsl <= 7): q = rint(y * 2^(8 nsl - 1)) as nsl balanced digits d_t in [-128, 127], the leading one
+// in [-64, 64] (|q| <= 2^(8 nsl - 2)).  Adding 128 to every byte makes them plain bytes: q + B = sum (d_t + 128) 256^..
+__device__ __forceinline__ void ozaki_digits256(double ys, int nsl, int d[MCD_OZAKI_MAX_SLICES]) {
+  const long long q = __double2ll_rn(ys);
+  const unsigned long long B = 0x8080808080808080ull & ((1ull << (8 * nsl)) - 1ull);
+  const unsigned long long qb = (unsigned long long)q + B;
+#pragma unroll
+  for (int t = 0; t < MCD_OZAKI_MAX_SLICES; ++t)
+    d[t] = (t < nsl) ? (int)((qb >> (8 * (nsl - 1 - t))) & 255ull) - 128 : 0;
+}
+
+// digits of either radix, RB chosen at compile time (the generic kernels are instantiated per radix)
+template <int RB>
+__device__ __forceinline__ void ozaki_digits_of(double ys, int nsl, int d[MCD_OZAKI_MAX_SLICES]) {
+  if constexpr (RB == 8)
+    ozaki_digits256(ys, nsl, d);
+  else
+    ozaki_digits(ys, nsl, d);
+}
+
 // Split-precision operand for the tcgen05 path: y (|y| <= 1, a unit-norm centred value) is scaled by
 // 2^8 and written as fp16 hi + fp16 lo (22 significant bits; the scale keeps `lo` out of the fp16
 // subnormal range for every |y| > 5e-4).  hi*hi + hi*lo + lo*hi reproduces the product to ~2^-22.
@@ -101,7 +121,8 @@ __device__ __forceinline__ void split_fp16x2(double y, uint16_t& s0, uint16_t& s
 // gidx != nullptr: gene gather -- element g of the standardised row is X[row, gidx[g]] (the host only computes
 // the index arrays of the gene intersection, macrodna.py:89-91; the data never gets re-indexed on the host).
 // The row is then read with scattered 8-byte loads, but it is L1/L2 resident while its CTA works on it.
-template <int T, int NV, bool VEC>
+// RB: radix bits of the digit output (oz.rb), a template parameter so that each radix compiles to its own kernel.
+template <int T, int NV, bool VEC, int RB>
 __global__ void __launch_bounds__((T > 512 ? T : 512), 1)
 standardize_rows(const double* __restrict__ X, const int* __restrict__ gidx, int64_t ncells, int G, int64_t ldx,
                  double* __restrict__ Y,
@@ -174,17 +195,17 @@ standardize_rows(const double* __restrict__ X, const int* __restrict__ gidx, int
     if (umax > 0.0 && isfinite(umax)) (void)frexp(umax, &ex);  // umax = f * 2^ex, f in [0.5, 1)
     const int e = -ex - 1;
     if (t == 0) oz.scale[row] = scalbn(1.0, -e);
-    // one multiplier per row: 1/nrm times the exact power of two 2^(e + 7 nsl - 1)  (bit-identical to scaling
+    // one multiplier per row: 1/nrm times the exact power of two 2^(e + rb nsl - 1)  (bit-identical to scaling
     // the rounded quotient afterwards: a power-of-two factor commutes with rounding)
-    const double mul = inv * scalbn(1.0, e + 7 * oz.nsl - 1);
+    const double mul = inv * scalbn(1.0, e + RB * oz.nsl - 1);
     int8_t* o = oz.digits + row * oz.ldk8;
 #pragma unroll
     for (int k = 0; k < NV; ++k) {
       const int g = 2 * (t + k * T);
       if (g < G) {
         int d0[MCD_OZAKI_MAX_SLICES], d1[MCD_OZAKI_MAX_SLICES];
-        ozaki_digits(v[k].x * mul, oz.nsl, d0);
-        ozaki_digits((g + 1 < G) ? v[k].y * mul : 0.0, oz.nsl, d1);
+        ozaki_digits_of<RB>(v[k].x * mul, oz.nsl, d0);
+        ozaki_digits_of<RB>((g + 1 < G) ? v[k].y * mul : 0.0, oz.nsl, d1);
 #pragma unroll
         for (int sl = 0; sl < MCD_OZAKI_MAX_SLICES; ++sl)
           if (sl < oz.nsl)  // g is even and ldk8 a multiple of 64: aligned 2-byte store
@@ -246,7 +267,9 @@ standardize_rows(const double* __restrict__ X, const int* __restrict__ gidx, int
 //     1.5 * 2^52 + B (B = 64 in every 7-bit field): the low mantissa bits of the result are q + B
 //     (NSL <= 7: |q + B| < 2^51; 8 slices need 56 bits and keep cvt.rni.s64);
 //   * bytes are packed with PRMT, and  ((w & 0x7f7f7f7f) + 0x40404040) ^ 0x80808080  turns the four biased
-//     fields d + 64 into the int8 digits d  (no carry can cross a byte: d + 128 <= 191).
+//     fields d + 64 into the int8 digits d  (no carry can cross a byte: d + 128 <= 191);
+//   * radix-256 digits (RB = 8) are whole bytes of q + B (B = 128 in every byte): PRMT and one XOR, see
+//     ozaki_store_slices256.
 template <int NSL>
 __device__ __forceinline__ void ozaki_bits(double c, double mul, double magic, uint32_t& lo, uint32_t& hi) {
   if (NSL <= 7) {
@@ -286,11 +309,27 @@ __device__ __forceinline__ void ozaki_store_slices(const uint32_t (&lo)[4], cons
   }
 }
 
+// Radix-256 digits (NSL <= 6, the magic constant then carries B = 0x80 in every byte): the digit of slice SL is byte
+// 8 (NSL-1-SL) of q + B, so PRMT gathers it from the four genes as it stands and  ^ 0x80808080  turns the biased
+// bytes d + 128 into the int8 digits d.  No masks, no field shifts.
+template <int NSL, int SL>
+__device__ __forceinline__ void ozaki_store_slices256(const uint32_t (&lo)[4], const uint32_t (&hi)[4], int8_t* o,
+                                                      int64_t slice_stride) {
+  if constexpr (SL < NSL) {
+    constexpr int BYTE = NSL - 1 - SL;  // byte of the 64-bit q + B
+    constexpr uint32_t SEL = (uint32_t)(BYTE & 3) | ((uint32_t)(4 + (BYTE & 3)) << 4);
+    const uint32_t w01 = BYTE < 4 ? __byte_perm(lo[0], lo[1], SEL) : __byte_perm(hi[0], hi[1], SEL);
+    const uint32_t w23 = BYTE < 4 ? __byte_perm(lo[2], lo[3], SEL) : __byte_perm(hi[2], hi[3], SEL);
+    *reinterpret_cast<uint32_t*>(o + SL * slice_stride) = __byte_perm(w01, w23, 0x5410) ^ 0x80808080u;
+    ozaki_store_slices256<NSL, SL + 1>(lo, hi, o, slice_stride);
+  }
+}
+
 // T threads per row, NV4 sweeps of 4 genes per thread (row capacity 4*T*NV4 >= ldk8), digit output only.
 // vec: X is 32-byte aligned and ldx a multiple of 4 (256-bit loads legal).
 // Everything of the digit pass behind the load: v holds the row slice of this thread (4 consecutive genes per k),
 // sum its partial sum.  Shared by the one-row-per-launch-CTA kernel and the persistent streaming kernel below.
-template <int T, int NV4, int NSL>
+template <int T, int NV4, int NSL, int RB>
 __device__ __forceinline__ void digits_row_finish(double (&v)[NV4][4], double sum, int t, int64_t row, bool live, int G,
                                                   double* __restrict__ norms, int* __restrict__ flags,
                                                   const mcd_ozaki_out& oz, double* red) {
@@ -336,8 +375,10 @@ __device__ __forceinline__ void digits_row_finish(double (&v)[NV4][4], double su
   if (umax > 0.0 && isfinite(umax)) (void)frexp(umax, &ex);
   const int sh = -ex - 1;
   if (t == 0) oz.scale[row] = scalbn(1.0, -sh);
-  const double mul = inv * scalbn(1.0, sh + 7 * NSL - 1);
-  const unsigned long long B = (0x0102040810204081ull << 6) & ((1ull << (7 * NSL)) - 1ull);
+  static_assert(RB == 7 || (RB == 8 && NSL <= 6), "radix-256 digits need B < 2^51");
+  const double mul = inv * scalbn(1.0, sh + RB * NSL - 1);
+  const unsigned long long B = RB == 8 ? 0x8080808080808080ull >> (64 - 8 * NSL)
+                                       : (0x0102040810204081ull << 6) & ((1ull << (7 * NSL)) - 1ull);
   const double magic = 6755399441055744.0 + (double)B;  // 1.5 * 2^52 + B, exact (B < 2^51 when NSL <= 7)
   int8_t* o = oz.digits + row * oz.ldk8 + 4 * t;
   const int ldk8 = (int)oz.ldk8;
@@ -348,13 +389,16 @@ __device__ __forceinline__ void digits_row_finish(double (&v)[NV4][4], double su
       uint32_t lo[4], hi[4];
 #pragma unroll
       for (int i = 0; i < 4; ++i) ozaki_bits<NSL>(v[k][i], mul, magic, lo[i], hi[i]);
-      ozaki_store_slices<NSL, 0>(lo, hi, o + 4 * k * T, oz.slice_stride);
+      if constexpr (RB == 8)
+        ozaki_store_slices256<NSL, 0>(lo, hi, o + 4 * k * T, oz.slice_stride);
+      else
+        ozaki_store_slices<NSL, 0>(lo, hi, o + 4 * k * T, oz.slice_stride);
     }
   }
 }
 
 
-template <int T, int NV4, int NSL>
+template <int T, int NV4, int NSL, int RB>
 __global__ void __launch_bounds__(512, 1)
 standardize_digits(const double* __restrict__ X, const int* __restrict__ gidx, int64_t ncells, int G, int64_t ldx,
                    int vec, double* __restrict__ norms, int* __restrict__ flags, const mcd_ozaki_out oz) {
@@ -395,7 +439,7 @@ standardize_digits(const double* __restrict__ X, const int* __restrict__ gidx, i
     v[k][3] = a3;
     sum += (a0 + a1) + (a2 + a3);
   }
-  digits_row_finish<T, NV4, NSL>(v, sum, t, row, live, G, norms, flags, oz, red);
+  digits_row_finish<T, NV4, NSL, RB>(v, sum, t, row, live, G, norms, flags, oz, red);
 }
 
 // Persistent streaming form for long rows (T = 512: one row per CTA at a time).  The one-row-per-CTA kernel above
@@ -405,7 +449,7 @@ standardize_digits(const double* __restrict__ X, const int* __restrict__ gidx, i
 // cp.async.bulk) of the whole row, completion on an mbarrier -- while the current row is reduced, turned into digit
 // slices and stored from registers.  Same thread <-> gene mapping and the same arithmetic as above: bit-identical.
 // Needs X 16-byte aligned, ldx and G even (bulk copies move multiples of 16 bytes) and no gene gather.
-template <int NV4, int NSL>
+template <int NV4, int NSL, int RB>
 __global__ void __launch_bounds__(512, 1)
 standardize_digits_stream(const double* __restrict__ X, int64_t ncells, int G, int64_t ldx, double* __restrict__ norms,
                           int* __restrict__ flags, const mcd_ozaki_out oz) {
@@ -474,13 +518,13 @@ standardize_digits_stream(const double* __restrict__ X, int64_t ncells, int G, i
                    "l"(X + nxt * ldx), "r"(bytes), "r"(bar_a)
                    : "memory");
     }
-    digits_row_finish<T, NV4, NSL>(v, sum, t, row, true, G, norms, flags, oz, red);
+    digits_row_finish<T, NV4, NSL, RB>(v, sum, t, row, true, G, norms, flags, oz, red);
   }
 }
 
-template <int T, int NV4>
-int launch_digits(mcd_context* h, const double* X, const int* gidx, int64_t ncells, int G, int64_t ldx, double* norms,
-                  const mcd_ozaki_out& oz) {
+template <int T, int NV4, int NSL, int RB>
+int launch_digits_fmt(mcd_context* h, const double* X, const int* gidx, int64_t ncells, int G, int64_t ldx, double* norms,
+                      const mcd_ozaki_out& oz) {
   constexpr int ROWS = 512 / T;
   const unsigned grid = (unsigned)((ncells + ROWS - 1) / ROWS);
   const int vec = ((reinterpret_cast<uintptr_t>(X) & 31) == 0) && ((ldx & 3) == 0);
@@ -489,26 +533,33 @@ int launch_digits(mcd_context* h, const double* X, const int* gidx, int64_t ncel
     // long rows, plenty of them: persistent CTAs with the next row prefetched by a bulk copy
     const size_t smem = ((size_t)G * 8 + 127) / 128 * 128;
     const unsigned pgrid = (unsigned)h->sm_count;
-    if (oz.nsl == 6) {
-      MCD_CUDA(h, cudaFuncSetAttribute(standardize_digits_stream<NV4, 6>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      standardize_digits_stream<NV4, 6><<<pgrid, 512, smem, h->stream>>>(X, ncells, G, ldx, norms, h->d_flags, oz);
-    } else {
-      MCD_CUDA(h, cudaFuncSetAttribute(standardize_digits_stream<NV4, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      standardize_digits_stream<NV4, 8><<<pgrid, 512, smem, h->stream>>>(X, ncells, G, ldx, norms, h->d_flags, oz);
-    }
+    MCD_CUDA(h, cudaFuncSetAttribute(standardize_digits_stream<NV4, NSL, RB>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                     (int)smem));
+    standardize_digits_stream<NV4, NSL, RB><<<pgrid, 512, smem, h->stream>>>(X, ncells, G, ldx, norms, h->d_flags, oz);
     MCD_LAUNCH_CHECK(h, "standardize_digits_stream");
     return MCD_OK;
   }
-  if (oz.nsl == 6)
-    standardize_digits<T, NV4, 6><<<grid, 512, 0, h->stream>>>(X, gidx, ncells, G, ldx, vec, norms, h->d_flags, oz);
-  else
-    standardize_digits<T, NV4, 8><<<grid, 512, 0, h->stream>>>(X, gidx, ncells, G, ldx, vec, norms, h->d_flags, oz);
+  standardize_digits<T, NV4, NSL, RB><<<grid, 512, 0, h->stream>>>(X, gidx, ncells, G, ldx, vec, norms, h->d_flags, oz);
   MCD_LAUNCH_CHECK(h, "standardize_digits");
   return MCD_OK;
 }
 
+// the digit formats the fast path is compiled for: radix 128 x 6 or 8 slices, radix 256 x 5 (mcd_ozaki_format)
+bool fast_digit_format(const mcd_ozaki_out& oz) {
+  return (oz.rb == 7 && (oz.nsl == 6 || oz.nsl == 8)) || (oz.rb == 8 && oz.nsl == 5);
+}
+
+template <int T, int NV4>
+int launch_digits(mcd_context* h, const double* X, const int* gidx, int64_t ncells, int G, int64_t ldx, double* norms,
+                  const mcd_ozaki_out& oz) {
+  if (oz.rb == 8) return launch_digits_fmt<T, NV4, 5, 8>(h, X, gidx, ncells, G, ldx, norms, oz);
+  if (oz.nsl == 6) return launch_digits_fmt<T, NV4, 6, 7>(h, X, gidx, ncells, G, ldx, norms, oz);
+  return launch_digits_fmt<T, NV4, 8, 7>(h, X, gidx, ncells, G, ldx, norms, oz);
+}
+
 // Rows longer than the register-resident capacity: one 512-thread block per row, three sweeps
 // (the row stays L2-resident between sweeps; declared as a 3-read variant in DESIGN.md).
+template <int RB>
 __global__ void __launch_bounds__(512)
 standardize_rows_long(const double* __restrict__ X, const int* __restrict__ gidx, int64_t ncells, int64_t G,
                       int64_t ldx, double* __restrict__ Y,
@@ -550,11 +601,11 @@ standardize_rows_long(const double* __restrict__ X, const int* __restrict__ gidx
     if (umax > 0.0 && isfinite(umax)) (void)frexp(umax, &ex);
     const int sh = -ex - 1;
     if (threadIdx.x == 0) oz.scale[row] = scalbn(1.0, -sh);
-    const double mul = inv1 * scalbn(1.0, sh + 7 * oz.nsl - 1);
+    const double mul = inv1 * scalbn(1.0, sh + RB * oz.nsl - 1);
     int8_t* o = oz.digits + row * oz.ldk8;
     for (int64_t e = threadIdx.x; e < oz.ldk8; e += 512) {
       int d[MCD_OZAKI_MAX_SLICES];
-      ozaki_digits(e < G ? (at(e) - mean) * mul : 0.0, oz.nsl, d);
+      ozaki_digits_of<RB>(e < G ? (at(e) - mean) * mul : 0.0, oz.nsl, d);
 #pragma unroll
       for (int sl = 0; sl < MCD_OZAKI_MAX_SLICES; ++sl)
         if (sl < oz.nsl) o[sl * oz.slice_stride + e] = (int8_t)d[sl];
@@ -579,12 +630,16 @@ int launch_t(mcd_context* h, bool vec, const double* X, const int* gidx, int64_t
   constexpr int BLOCK = (T > 512 ? T : 512);
   constexpr int ROWS = BLOCK / T;
   const int64_t grid = (ncells + ROWS - 1) / ROWS;
-  if (vec)
-    standardize_rows<T, NV, true><<<(unsigned)grid, BLOCK, 0, h->stream>>>(X, gidx, ncells, G, ldx, Y, ldk, S, S_lo,
-                                                                          ldk16, norms, h->d_flags, oz);
+  // radix-256 digits come here only off the fast path (mcd_launch_standardize): scalar loads suffice
+  if (oz.digits != nullptr && oz.rb == 8)
+    standardize_rows<T, NV, false, 8><<<(unsigned)grid, BLOCK, 0, h->stream>>>(X, gidx, ncells, G, ldx, Y, ldk, S, S_lo,
+                                                                              ldk16, norms, h->d_flags, oz);
+  else if (vec)
+    standardize_rows<T, NV, true, 7><<<(unsigned)grid, BLOCK, 0, h->stream>>>(X, gidx, ncells, G, ldx, Y, ldk, S, S_lo,
+                                                                             ldk16, norms, h->d_flags, oz);
   else
-    standardize_rows<T, NV, false><<<(unsigned)grid, BLOCK, 0, h->stream>>>(X, gidx, ncells, G, ldx, Y, ldk, S, S_lo,
-                                                                           ldk16, norms, h->d_flags, oz);
+    standardize_rows<T, NV, false, 7><<<(unsigned)grid, BLOCK, 0, h->stream>>>(X, gidx, ncells, G, ldx, Y, ldk, S, S_lo,
+                                                                              ldk16, norms, h->d_flags, oz);
   MCD_LAUNCH_CHECK(h, "standardize_rows");
   return MCD_OK;
 }
@@ -599,7 +654,7 @@ int mcd_launch_standardize(mcd_context* h, const double* X, int64_t ncells, int6
   if (ozaki != nullptr) oz = *ozaki;
   const bool vec = ((reinterpret_cast<uintptr_t>(X) & 15) == 0) && ((ldx & 1) == 0);
   const int g = (int)G;
-  if (oz.digits != nullptr && centred == nullptr && slices == nullptr && (oz.nsl == 6 || oz.nsl == 8) &&
+  if (oz.digits != nullptr && centred == nullptr && slices == nullptr && fast_digit_format(oz) &&
       oz.ldk8 <= 24576 && (oz.ldk8 & 3) == 0 && (oz.slice_stride & 3) == 0 &&
       (reinterpret_cast<uintptr_t>(oz.digits) & 3) == 0 && !h->opt.k1_generic) {
     const int64_t cap = oz.ldk8;  // the sweeps also write the zero padding up to ldk8
@@ -620,8 +675,12 @@ int mcd_launch_standardize(mcd_context* h, const double* X, int64_t ncells, int6
   if (G <= 16384) return launch_t<512, 16>(h, vec, X, gidx, ncells, g, ldx, centred, ldk, slices, slices_lo, ldk16, norms, oz);
   if (G <= 20480) return launch_t<512, 20>(h, vec, X, gidx, ncells, g, ldx, centred, ldk, slices, slices_lo, ldk16, norms, oz);
   if (G <= 24576) return launch_t<512, 24>(h, vec, X, gidx, ncells, g, ldx, centred, ldk, slices, slices_lo, ldk16, norms, oz);
-  standardize_rows_long<<<(unsigned)ncells, 512, 0, h->stream>>>(X, gidx, ncells, G, ldx, centred, ldk, slices,
-                                                                slices_lo, ldk16, norms, h->d_flags, oz);
+  if (oz.digits != nullptr && oz.rb == 8)
+    standardize_rows_long<8><<<(unsigned)ncells, 512, 0, h->stream>>>(X, gidx, ncells, G, ldx, centred, ldk, slices,
+                                                                     slices_lo, ldk16, norms, h->d_flags, oz);
+  else
+    standardize_rows_long<7><<<(unsigned)ncells, 512, 0, h->stream>>>(X, gidx, ncells, G, ldx, centred, ldk, slices,
+                                                                     slices_lo, ldk16, norms, h->d_flags, oz);
   MCD_LAUNCH_CHECK(h, "standardize_rows_long");
   return MCD_OK;
 }

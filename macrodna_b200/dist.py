@@ -64,9 +64,10 @@ class ShardedCell2Cell:
         self.world, self.rank, self.device = world, rank, device
         self.precision = precision
         if precision == "ozaki":
-            # exact int32 accumulation bounds the gene count of the integer path (as in the fused single-GPU driver)
-            nsl = int(handle.lib.mcd_ozaki_slices(handle.h, M, N, G))
-            if nsl * 4096.0 * handle.lib.mcd_padded_k_split(G) >= 2147483648.0:
+            # the digit format of the fused single-GPU driver; exact int32 accumulation bounds the gene count of the
+            # integer path, longer rows take the FP64 pipe there too
+            self.nsl, self.rb, exact = handle.ozaki_format(M, N, G)
+            if not exact:
                 self.precision = "fp64"
         self.lo, self.hi = row_shard(M, world, rank)
         self._bufs = None
@@ -92,7 +93,7 @@ class ShardedCell2Cell:
                 ops = dict(a=torch.empty((m_loc, ldk), **f64), b=torch.empty((self.N, ldk), **f64))
             elif self.precision == "ozaki":
                 ldk = lib.mcd_padded_k_split(self.G)
-                nsl = int(lib.mcd_ozaki_slices(self.h.h, self.M, self.N, self.G))
+                nsl = self.nsl
                 i8 = dict(dtype=torch.int8, device=self.device)
                 ops = dict(a=torch.empty((nsl, m_loc, ldk), **i8), b=torch.empty((nsl, self.N, ldk), **i8),
                            sa=torch.empty(m_loc, **f64), sb=torch.empty(self.N, **f64), nsl=nsl)
@@ -120,11 +121,11 @@ class ShardedCell2Cell:
             events[1].record(ext)
             chk(lib.mcd_corr_fp64(h, pa, m_loc, pb, N, G, ldk, na, nb, c, ldc, None, 0))
         elif self.precision == "ozaki":
-            sa, sb, nsl = b["sa"].data_ptr(), b["sb"].data_ptr(), b["nsl"]
-            chk(lib.mcd_standardize_ozaki(h, rna_loc.data_ptr(), m_loc, G, G, pa, nsl, sa, na))
-            chk(lib.mcd_standardize_ozaki(h, dna.data_ptr(), N, G, G, pb, nsl, sb, nb))
+            sa, sb, nsl, rb = b["sa"].data_ptr(), b["sb"].data_ptr(), b["nsl"], self.rb
+            chk(lib.mcd_standardize_ozaki_radix(h, rna_loc.data_ptr(), m_loc, G, G, pa, nsl, rb, sa, na))
+            chk(lib.mcd_standardize_ozaki_radix(h, dna.data_ptr(), N, G, G, pb, nsl, rb, sb, nb))
             events[1].record(ext)
-            chk(lib.mcd_corr_ozaki(h, pa, m_loc, pb, N, G, ldk, nsl, sa, sb, na, nb, c, ldc, None, 0))
+            chk(lib.mcd_corr_ozaki_radix(h, pa, m_loc, pb, N, G, ldk, nsl, rb, sa, sb, na, nb, c, ldc, None, 0))
         else:
             chk(lib.mcd_standardize_split(h, rna_loc.data_ptr(), m_loc, G, G, pa, na))
             chk(lib.mcd_standardize_split(h, dna.data_ptr(), N, G, G, pb, nb))
