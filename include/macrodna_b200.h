@@ -12,7 +12,8 @@
  * mcd_last_error(h) gives the detail string of the last failure on a handle.
  * The caller owns every buffer it passes.  A handle is bound to one CUDA device
  * and one stream; calls on one handle are serialised by the caller; distinct
- * handles are independent (no global state).
+ * handles are independent (the only process-wide state is the counter that
+ * numbers the runs, see mcd_share_resident).
  */
 #ifndef MACRODNA_B200_H
 #define MACRODNA_B200_H
@@ -325,6 +326,48 @@ int mcd_loo_sweep(mcd_handle h, const int32_t* cells, int64_t ncells, int64_t k_
                   double* test_corr, double* total, int32_t* assign, int32_t* step, double* step_obj, double* match_corr,
                   double* cert_gap, int concurrency, mcd_stats* stats);
 int mcd_corr_rows(mcd_handle h, const int32_t* rows, int64_t nrows, double* out, int out_space);
+
+/*
+ * Views on several GPUs of one node, from one caller.  hs[0..ndev) are distinct handles (one context named twice
+ * returns MCD_ERR_INVALID; separate contexts on one device are allowed).
+ *
+ * mcd_share_resident: copies the correlation matrix resident on hs[0] into hs[1..ndev) -- peer copies between devices
+ * (NVLink), a device-to-device copy for a handle on hs[0]'s device.  A copy is a resident matrix WITHOUT an
+ * assignment: the view calls above (mcd_subinstance_steps, the sweeps, the null test, mcd_corr_rows, mcd_corr_pairs)
+ * run on it, mcd_last_match_values refuses it.  Generations: every successful mcd_cell2cell / mcd_cell2cell_gather /
+ * mcd_cell2cell_multi run gives the handle's matrix a new id, unique in the process; a copy carries the id of the run
+ * it copied.  Every _multi call below requires that hs[1..) hold a copy of hs[0]'s CURRENT generation with the same
+ * M and N, and returns MCD_ERR_INVALID otherwise: call mcd_share_resident again after every run on hs[0] (a run on
+ * any of the handles, mcd_cell2cell_multi included, drops the copies it overwrites).  hs[0]'s matrix, its
+ * assignment and mcd_last_match_values are unchanged by all of these calls.
+ *
+ * mcd_subinstance_sweep_multi / mcd_loo_sweep_multi: arguments after the handle list and outputs (HOST) as
+ * mcd_subinstance_sweep / mcd_loo_sweep; ndev == 1 is exactly the single-handle call.  Replicates are dealt in
+ * contiguous batches over the handles (one host thread per handle, `concurrency` workers on each), with hs[0]'s
+ * solver options on every handle.  Each worker gets the cooperative grid of a single-handle call with the same
+ * `concurrency` on its own device, so a replicate follows the same solver trajectory whichever device (of one kind)
+ * solves it: every output is bit-identical to the single-handle call where the replicate's optimum is unique (no
+ * duplicated DNA cells); with exact ties the objectives agree and the assignment is one of the optima.  A replicate
+ * re-solved without the class treatment of duplicated cells is re-solved on the handle that owned it.  stats: counters
+ * and sweep_fallbacks summed over the handles, cert_rel_gap / cert_max_violation the maximum, kernel_launches over
+ * every handle and worker, the per-step arrays those of the handle that solved the last batch, ms_total / ms_lap the
+ * host wall time from the first enqueue to the last synchronise (events of different devices are not comparable).
+ *
+ * mcd_null_assignments_multi: the trials are split into contiguous ranges, one per handle in proportion to its SM
+ * count (a handle may get none); each device computes trials [t0, t0 + n) of the draw defined at
+ * mcd_null_assignments.  A trial depends only on (seed, t, C), so sums / medians (HOST, medians may be NULL) are
+ * bit-identical to mcd_null_assignments on hs[0].
+ * Measured throughput: DESIGN.md section 5b (over several GPUs: not measured).
+ */
+int mcd_share_resident(mcd_handle* hs, int ndev);
+int mcd_subinstance_sweep_multi(mcd_handle* hs, int ndev, int64_t nrep, const int32_t* rna_rows, int64_t m_sub,
+                                const int32_t* dna_cols, int64_t n_sub, int32_t* assign, int32_t* step,
+                                double* step_obj, double* cert_gap, int concurrency, mcd_stats* stats);
+int mcd_loo_sweep_multi(mcd_handle* hs, int ndev, const int32_t* cells, int64_t ncells, int64_t k_steps,
+                        int32_t* test_col, double* test_corr, double* total, int32_t* assign, int32_t* step,
+                        double* step_obj, double* match_corr, double* cert_gap, int concurrency, mcd_stats* stats);
+int mcd_null_assignments_multi(mcd_handle* hs, int ndev, int64_t trials, uint64_t seed, double* sums,
+                               double* medians);
 /* out[k] = C[rows[k], cols[k]] of the resident matrix (HOST indices, HOST out): the `corr_val` of a sub-instance's
  * matched pairs (run_loo_experiment.py:285). */
 int mcd_corr_pairs(mcd_handle h, const int32_t* rows, const int32_t* cols, int64_t n, double* out);

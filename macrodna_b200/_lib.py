@@ -107,6 +107,12 @@ SIGNATURES = {
     "mcd_corr_rows": (_I, [_VP, _VP, _I64, _VP, _I]),
     "mcd_corr_pairs": (_I, [_VP, _VP, _VP, _I64, _VP]),
     "mcd_null_assignments": (_I, [_VP, _I64, C.c_uint64, _VP, _VP, _I]),
+    "mcd_share_resident": (_I, [C.POINTER(_VP), _I]),
+    "mcd_subinstance_sweep_multi": (_I, [C.POINTER(_VP), _I, _I64, _VP, _I64, _VP, _I64, _VP, _VP, _VP, _VP, _I,
+                                         C.POINTER(McdStats)]),
+    "mcd_loo_sweep_multi": (_I, [C.POINTER(_VP), _I, _VP, _I64, _I64, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _I,
+                                 C.POINTER(McdStats)]),
+    "mcd_null_assignments_multi": (_I, [C.POINTER(_VP), _I, _I64, C.c_uint64, _VP, _VP]),
     "mcd_lap_steps": (_I, [_VP, _VP, _I64, _VP, _I64, _I64, _I64, _VP, _VP, _VP, _I, C.POINTER(McdStats)]),
     "mcd_cell2cell_gather": (
         _I,
@@ -206,6 +212,57 @@ def cell2cell_multi(handles, rna, dna, M, N, G, ld_rna=None, ld_dna=None, precis
                                     C.byref(stats))
     h0.check(st)
     return assign, step, step_obj, stats
+
+
+def _handle_array(handles):
+    """The ``mcd_handle*`` of a multi-handle call.  An empty list, or one context listed twice (two host threads would
+    drive it at once), is refused here, before any GPU call."""
+    handles = list(handles)
+    if not handles:
+        raise ValueError("macrodna_b200: at least one handle is required")
+    if len({id(h) for h in handles}) != len(handles):
+        raise ValueError("macrodna_b200: a handle is listed twice (list a device twice to get separate contexts on it)")
+    return handles, (C.c_void_p * len(handles))(*[h.h for h in handles])
+
+
+def share_resident(handles):
+    """Copy the correlation matrix resident on ``handles[0]`` to every other handle (``mcd_share_resident``): the
+    copies let the ``*_multi`` view calls deal their work over all of them.  A copy is valid until the next run on
+    ``handles[0]``; a copy carries no assignment (``last_match_values`` refuses it)."""
+    handles, arr = _handle_array(handles)
+    for h in handles[1:]:
+        h.resident_token = None
+    handles[0].check(handles[0].lib.mcd_share_resident(arr, len(handles)))
+    for h in handles[1:]:
+        h.resident_token = handles[0].resident_token  # the same run's matrix
+
+
+def subinstance_sweep_multi(handles, dna_cols, rna_rows=None, M=None, concurrency=8):
+    """:meth:`Handle.subinstance_sweep` with the replicates dealt over ``handles`` (``mcd_subinstance_sweep_multi``;
+    ``handles[1:]`` hold copies of ``handles[0]``'s matrix, see :func:`share_resident`)."""
+    handles, arr = _handle_array(handles)
+    h0 = handles[0]
+    return h0._subinstance_sweep(lambda *a: h0.lib.mcd_subinstance_sweep_multi(arr, len(handles), *a), dna_cols,
+                                 rna_rows, M, concurrency)
+
+
+def loo_sweep_multi(handles, cells, k_steps, M, N, full=False, concurrency=8):
+    """:meth:`Handle.loo_sweep` with the replicates dealt over ``handles`` (``mcd_loo_sweep_multi``)."""
+    handles, arr = _handle_array(handles)
+    h0 = handles[0]
+    return h0._loo_sweep(lambda *a: h0.lib.mcd_loo_sweep_multi(arr, len(handles), *a), cells, k_steps, M, N, full,
+                         concurrency)
+
+
+def null_assignments_multi(handles, trials, seed=2023, medians=False):
+    """:meth:`Handle.null_assignments` with the trials split over ``handles`` (``mcd_null_assignments_multi``): bit
+    for bit what ``handles[0]`` alone returns."""
+    handles, arr = _handle_array(handles)
+    h0 = handles[0]
+    sums = np.empty(int(trials), dtype=np.float64)
+    med = np.empty(int(trials), dtype=np.float64) if medians else None
+    h0.check(h0.lib.mcd_null_assignments_multi(arr, len(handles), int(trials), int(seed), _ptr(sums), _ptr(med)))
+    return (sums, med) if medians else sums
 
 
 class Handle:
@@ -337,6 +394,10 @@ class Handle:
         """``len(dna_cols)`` replicates of :meth:`subinstance` kept ``concurrency`` at a time in flight
         (``mcd_subinstance_sweep``).  ``dna_cols``: int array [nrep, n_sub] of columns of the resident matrix
         (repeats allowed).  Returns (assign [nrep, m], step [nrep, m], objs [nrep, nsteps], cert_gap [nrep], stats)."""
+        return self._subinstance_sweep(lambda *a: self.lib.mcd_subinstance_sweep(self.h, *a), dna_cols, rna_rows, M,
+                                       concurrency)
+
+    def _subinstance_sweep(self, call, dna_cols, rna_rows, M, concurrency):
         dna_cols = np.ascontiguousarray(dna_cols, dtype=np.int32)
         if dna_cols.ndim != 2:
             raise ValueError("dna_cols must be a 2-D array [replicates, DNA cells per replicate]")
@@ -352,8 +413,8 @@ class Handle:
         objs = np.empty((nrep, nsteps), dtype=np.float64)
         gaps = np.empty(nrep, dtype=np.float64)
         stats = McdStats()
-        self.check(self.lib.mcd_subinstance_sweep(self.h, nrep, _ptr(rna_rows), m, _ptr(dna_cols), n, _ptr(assign),
-                                                  _ptr(step), _ptr(objs), _ptr(gaps), int(concurrency), C.byref(stats)))
+        self.check(call(nrep, _ptr(rna_rows), m, _ptr(dna_cols), n, _ptr(assign), _ptr(step), _ptr(objs), _ptr(gaps),
+                        int(concurrency), C.byref(stats)))
         return assign, step, objs, gaps, stats
 
     def loo_sweep(self, cells, k_steps, M, N, full=False, concurrency=8):
@@ -361,6 +422,9 @@ class Handle:
         Returns (dict of arrays, stats): ``test_col`` [ncells] (-1: no eligible column), ``test_corr``, ``total``,
         ``cert_gap``; with ``full`` also ``assign`` / ``step`` / ``match_corr`` [ncells, M-1] and ``step_obj``
         [ncells, nsteps]."""
+        return self._loo_sweep(lambda *a: self.lib.mcd_loo_sweep(self.h, *a), cells, k_steps, M, N, full, concurrency)
+
+    def _loo_sweep(self, call, cells, k_steps, M, N, full, concurrency):
         cells = np.ascontiguousarray(cells, dtype=np.int32).ravel()
         n, m = cells.size, int(M) - 1
         nsteps = self.lib.mcd_num_steps(m, int(N))
@@ -370,10 +434,9 @@ class Handle:
             out.update(assign=np.empty((n, m), dtype=np.int32), step=np.empty((n, m), dtype=np.int32),
                        step_obj=np.empty((n, nsteps), dtype=np.float64), match_corr=np.empty((n, m), dtype=np.float64))
         stats = McdStats()
-        self.check(self.lib.mcd_loo_sweep(self.h, _ptr(cells), n, int(k_steps), _ptr(out["test_col"]),
-                                          _ptr(out["test_corr"]), _ptr(out["total"]), _ptr(out.get("assign")),
-                                          _ptr(out.get("step")), _ptr(out.get("step_obj")), _ptr(out.get("match_corr")),
-                                          _ptr(out["cert_gap"]), int(concurrency), C.byref(stats)))
+        self.check(call(_ptr(cells), n, int(k_steps), _ptr(out["test_col"]), _ptr(out["test_corr"]), _ptr(out["total"]),
+                        _ptr(out.get("assign")), _ptr(out.get("step")), _ptr(out.get("step_obj")),
+                        _ptr(out.get("match_corr")), _ptr(out["cert_gap"]), int(concurrency), C.byref(stats)))
         return out, stats
 
     def corr_rows(self, rows, N):

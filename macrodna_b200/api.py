@@ -56,6 +56,19 @@ def get_handles(devices) -> list:
     return out
 
 
+def _check_devices(devices):
+    """``devices=`` as a list of device ordinals (None stays None); refused before any GPU call if an entry is not a
+    non-negative integer."""
+    if devices is None:
+        return None
+    out = []
+    for d in devices:
+        if isinstance(d, bool) or not isinstance(d, (int, np.integer)) or d < 0:
+            raise ValueError("devices must be non-negative CUDA device ordinals, got %r" % (d,))
+        out.append(int(d))
+    return out
+
+
 class _StatsDict:
     """Merged stats of a two-call run, with the ``as_dict`` / attribute access of ``_lib.McdStats``."""
 
@@ -80,7 +93,9 @@ class MaCroDNA:
     ``clone`` and ``cell`` (``:14``).  Keyword-only extras default to reference behaviour:
 
     * ``devices``: list of CUDA devices of this node; more than one shards the correlation work by RNA rows
-      (``mcd_cell2cell_multi``), results identical to one device;
+      (``mcd_cell2cell_multi``), results identical to one device, and deals the replicates of
+      :meth:`leave_one_out_sweep` and :meth:`subinstance_sweep` over all of them (each device works on its own copy of
+      the correlation matrix, made on the first such call after a run);
     * ``precision``: ``"ozaki"`` (default: FP64-equivalent correlations from the int8 tcgen05 tensor cores, exact
       digit-slice products, ~1e-12 absolute), ``"fp64"`` (FP64 tensor pipe, DMMA) or ``"split"`` (tcgen05 fp16
       hi/lo split precision, ~3e-7 absolute);
@@ -104,7 +119,7 @@ class MaCroDNA:
         self.dna_label = dna_label
         # devices=[d0, d1, ...]: the RNA rows are sharded over these GPUs for standardisation + correlation (no exchange
         # inside the contraction), the shards meet on d0 over NVLink and d0 runs the step loop (mcd_cell2cell_multi)
-        self.devices = [int(d) for d in devices] if devices is not None else None
+        self.devices = _check_devices(devices)
         self.device = self.devices[0] if self.devices else device
         self.precision = precision
         self.clone_column = clone_column
@@ -309,15 +324,21 @@ class MaCroDNA:
             self._run()  # the reference recomputes `corrs` on every call anyway (run_loo_experiment.py:217-221)
         return h
 
-    def subinstance_assignment(self, rna_cells=None, dna_cells=None):
-        """Re-run the step loop on a replicate that only gathers cells of the frames of the last run: ``dna_cells``
-        may repeat and drop DNA cell ids (``new_dna = dna.loc[:, names]``, clonal_proportions_resampling.py:184-190;
-        run_dna_batch_removal_exp.py), ``rna_cells`` selects RNA cells.  The correlation matrix is NOT recomputed
-        (genes are untouched: the replicate's matrix is an index gather of the resident one).  Returns the
-        ``"resampling"`` frame ``[predicted_dna_cell, rna_cell, step]`` (clonal_proportions_resampling.py:166-169)."""
+    def _view_handles(self):
+        """The handles a sweep deals its replicates over: the one holding the resident matrix, then (``devices=`` with
+        more than one entry) one per further device holding a copy of it, made once per run."""
         h = self._ensure_resident()
+        if not self.devices or len(self.devices) < 2:
+            return [h]
+        hs = get_handles(self.devices)
+        if self._resident_token is None or any(x.resident_token is not self._resident_token for x in hs[1:]):
+            _lib.share_resident(hs)
+        return hs
+
+    def _sub_indices(self, rna_cells, dna_cells):
+        """Rows / columns of the resident matrix for a replicate of cell ids (None = all cells, in order), and the
+        selected ids."""
         all_rna, all_dna = self._resident_cells
-        M, N = self._resident_shape
         rows = cols = None
         sel_rna, sel_dna = all_rna, all_dna
         if rna_cells is not None:
@@ -327,15 +348,72 @@ class MaCroDNA:
                 raise ValueError("duplicate RNA cell ids")
             rows = np.array([pos[c] for c in sel_rna], dtype=np.int32)
         if dna_cells is not None:
-            pos = {}
-            for k, c in enumerate(all_dna):
-                pos.setdefault(c, k)
+            pos = self._dna_positions()
             sel_dna = list(dna_cells)
             cols = np.array([pos[c] for c in sel_dna], dtype=np.int32)
+        return rows, cols, sel_rna, sel_dna
+
+    def _dna_positions(self):
+        """DNA cell id -> column of the resident matrix (its first copy)."""
+        pos = {}
+        for k, c in enumerate(self._resident_cells[1]):
+            pos.setdefault(c, k)
+        return pos
+
+    def subinstance_assignment(self, rna_cells=None, dna_cells=None):
+        """Re-run the step loop on a replicate that only gathers cells of the frames of the last run: ``dna_cells``
+        may repeat and drop DNA cell ids (``new_dna = dna.loc[:, names]``, clonal_proportions_resampling.py:184-190;
+        run_dna_batch_removal_exp.py), ``rna_cells`` selects RNA cells.  The correlation matrix is NOT recomputed
+        (genes are untouched: the replicate's matrix is an index gather of the resident one).  Returns the
+        ``"resampling"`` frame ``[predicted_dna_cell, rna_cell, step]`` (clonal_proportions_resampling.py:166-169)."""
+        h = self._ensure_resident()
+        M, N = self._resident_shape
+        rows, cols, sel_rna, sel_dna = self._sub_indices(rna_cells, dna_cells)
         assign, step, objs, stats = h.subinstance(rows, cols, M=M, N=N)
         self.last_sub = {"assign": assign, "step": step, "objs": objs, "stats": stats.as_dict()}
         pred = [sel_dna[j] for j in assign.tolist()]
         return pd.DataFrame(list(zip(pred, sel_rna, step.tolist())), columns=["predicted_dna_cell", "rna_cell", "step"])
+
+    def subinstance_sweep(self, dna_cells_list, rna_cells=None, concurrency=8):
+        """Every replicate of ``dna_cells_list`` (each a list of DNA cell ids of the last run's frames, repeats and
+        omissions allowed) against the RNA cells ``rna_cells`` (None = all) in batched calls
+        (``mcd_subinstance_sweep``, ``concurrency`` solves in flight per device, over all of ``devices``): the
+        reference's resampling and DNA-removal sweeps (clonal_proportions_resampling.py:172-201,
+        run_dna_batch_removal_exp.py).  Returns the list of ``"resampling"`` frames a loop of
+        :meth:`subinstance_assignment` returns, frame for frame (replicates with duplicated DNA cells have exact ties:
+        any of the tied optima is returned, with the same objectives).  Per-replicate objectives, certificate gaps
+        and the stats go to ``self.last_sweep``."""
+        reps = [list(c) for c in dna_cells_list]
+        if not reps:
+            raise ValueError("dna_cells_list is empty")
+        if any(len(c) == 0 for c in reps):
+            raise ValueError("a replicate has no DNA cells")
+        hs = self._view_handles()
+        M, N = self._resident_shape
+        rows, _, sel_rna, _ = self._sub_indices(rna_cells, None)
+        m = M if rows is None else rows.size
+        pos = self._dna_positions()
+        cols = [np.array([pos[c] for c in rep], dtype=np.int32) for rep in reps]
+        # one batched call per replicate width (DNA-removal replicates may differ in size)
+        by_width = {}
+        for r, c in enumerate(cols):
+            by_width.setdefault(c.size, []).append(r)
+        frames = [None] * len(reps)
+        objs, gaps, stats = [None] * len(reps), np.empty(len(reps)), []
+        for idx in by_width.values():
+            block = np.stack([cols[r] for r in idx])
+            if len(hs) == 1:
+                a, s, o, g, st = hs[0].subinstance_sweep(block, rna_rows=rows, M=m, concurrency=concurrency)
+            else:
+                a, s, o, g, st = _lib.subinstance_sweep_multi(hs, block, rna_rows=rows, M=m, concurrency=concurrency)
+            stats.append(st.as_dict())
+            for k, r in enumerate(idx):
+                pred = [reps[r][j] for j in a[k].tolist()]
+                frames[r] = pd.DataFrame(list(zip(pred, sel_rna, s[k].tolist())),
+                                         columns=["predicted_dna_cell", "rna_cell", "step"])
+                objs[r], gaps[r] = o[k], g[k]
+        self.last_sweep = {"objs": objs, "cert_gap": gaps, "stats": stats}
+        return frames
 
     def leave_one_out(self, cell_idx, K_steps, biopsy_name=None):
         """run_loo_experiment.py:201-319.  The RNA cell at position ``cell_idx`` is removed, the step loop runs on the
@@ -417,10 +495,13 @@ class MaCroDNA:
             raise ValueError("leave_one_out_sweep: the DNA frame repeats cells with identical data (a resampled frame); "
                              "its correlation matrix is computed on the distinct cells, so leave-one-out replicates "
                              "cannot be taken from it -- pass the frame of distinct DNA cells")
-        h = self._ensure_resident()
+        hs = self._view_handles()
         rna_cells, dna_cells = self._resident_cells
         M, N = self._resident_shape
-        res, stats = h.loo_sweep(cells, K_steps, M, N, full=frames, concurrency=concurrency)
+        if len(hs) == 1:
+            res, stats = hs[0].loo_sweep(cells, K_steps, M, N, full=frames, concurrency=concurrency)
+        else:
+            res, stats = _lib.loo_sweep_multi(hs, cells, K_steps, M, N, full=frames, concurrency=concurrency)
         self.last_loo = {"cells": np.asarray(cells), "cert_gap": res["cert_gap"], "stats": stats.as_dict()}
         if frames:
             return [self._loo_frame(q, res["assign"][r], res["step"][r], res["match_corr"][r], res["step_obj"][r],
@@ -478,10 +559,12 @@ class random_test:
     the matched correlations of ONE random assignment like the reference, drawn from batches generated by
     ``mcd_null_assignments``; ``assign_many`` returns a whole batch (optionally with the medians of
     random_assignment_test_median.py).  Same distribution as the reference, not NumPy's random stream; every trial is
-    the draw written down at ``mcd_null_assignments`` (include/macrodna_b200.h), up to 2^24 cells a side."""
+    the draw written down at ``mcd_null_assignments`` (include/macrodna_b200.h), up to 2^24 cells a side.
+    ``devices=[d0, d1, ...]``: the trials are split over these GPUs (``mcd_null_assignments_multi``), bit for bit
+    the draws of one device."""
 
-    def __init__(self, rna_df=None, dna_df=None, *, device=0, precision="ozaki", seed=2023, batch=4096):
-        self._m = MaCroDNA(rna_df, dna_df, device=device, precision=precision)
+    def __init__(self, rna_df=None, dna_df=None, *, device=0, devices=None, precision="ozaki", seed=2023, batch=4096):
+        self._m = MaCroDNA(rna_df, dna_df, device=device, devices=devices, precision=precision)
         self._m._run()
         self.dna_cells, self.rna_cells = list(self._m._resident_cells[1]), list(self._m._resident_cells[0])
         M, N = self._m._resident_shape
@@ -490,8 +573,11 @@ class random_test:
         self._seed, self._batch, self._buf, self._pos, self._draws = int(seed), int(batch), None, 0, 0
 
     def assign_many(self, trials, seed=None, medians=False):
-        h = self._m._ensure_resident()
-        return h.null_assignments(trials, self._seed if seed is None else seed, medians=medians)
+        hs = self._m._view_handles()
+        seed = self._seed if seed is None else seed
+        if len(hs) == 1:
+            return hs[0].null_assignments(trials, seed, medians=medians)
+        return _lib.null_assignments_multi(hs, trials, seed, medians=medians)
 
     def assign(self):
         if self._buf is None or self._pos >= len(self._buf):

@@ -48,6 +48,27 @@ int mcd_ws(mcd_context* h, int slot, size_t bytes, void** out) {
   return MCD_OK;
 }
 
+// ------------------------------------------------------------------------------------------------
+// resident matrix: the correlation matrix of a handle's last run (with its assignment), or a copy of another handle's
+// (without one).  Generation ids are unique in the process, so equal ids mean "the same run's matrix".
+// ------------------------------------------------------------------------------------------------
+static std::atomic<uint64_t> g_generation(0);
+
+static bool has_matrix(const mcd_context* h) { return h->gen != 0 && h->last_M >= 1; }
+static bool has_assignment(const mcd_context* h) { return has_matrix(h) && h->last_assign != nullptr; }
+static void drop_resident(mcd_context* h) {
+  h->last_M = 0;
+  h->last_assign = nullptr;
+  h->gen = 0;
+}
+static void set_resident(mcd_context* h, int64_t M, int64_t N, int64_t ldc, const int* assign) {
+  h->last_M = M;
+  h->last_N = N;
+  h->last_ldc = ldc;
+  h->last_assign = assign;
+  h->gen = ++g_generation;
+}
+
 extern "C" {
 
 int mcd_abi_version(void) { return MCD_ABI_VERSION; }
@@ -805,8 +826,10 @@ int mcd_transpose_f64(mcd_handle h, const double* src, int64_t rows, int64_t col
 
 int mcd_last_match_values(mcd_handle h, double* out, int64_t M, int out_space) {
   if (!h) return MCD_ERR_INVALID;
-  if (!out || M < 1 || M != h->last_M || h->last_assign == nullptr)
-    return mcd_fail(h, MCD_ERR_INVALID, "mcd_last_match_values: no matching mcd_cell2cell result is resident");
+  if (!out || M < 1 || M != h->last_M || !has_assignment(h))
+    return mcd_fail(h, MCD_ERR_INVALID,
+                    "mcd_last_match_values: no matching mcd_cell2cell result is resident (a copy made by "
+                    "mcd_share_resident carries no assignment)");
   MCD_CUDA(h, cudaSetDevice(h->device));
   const double* C = static_cast<const double*>(h->ws[WS_C].ptr);
   double* tmp = out;
@@ -830,8 +853,7 @@ int mcd_lap_steps(mcd_handle h, const double* C, int64_t ldc, const double* Ct, 
   if (!C || !Ct || !assign || !step || M < 1 || N < 1 || ldc < N || ldct < M || M > 0x3fffffff || N > 0x3fffffff)
     return mcd_fail(h, MCD_ERR_INVALID, "mcd_lap_steps arguments");
   MCD_CUDA(h, cudaSetDevice(h->device));
-  h->last_M = 0;  // the resident cell2cell result (if any) is about to be overwritten
-  h->last_assign = nullptr;
+  drop_resident(h);  // the resident cell2cell result (if any) is about to be overwritten
   const int64_t nsteps = mcd_num_steps(M, N);
   void* misc = nullptr;
   int st = mcd_ws(h, WS_MISC, step_out_bytes(M, nsteps), &misc);
@@ -895,8 +917,7 @@ int mcd_cell2cell_gather(mcd_handle h, const double* rna, int64_t ld_rna, const 
   // exact int32 accumulation bounds the gene count of the integer path; longer rows use the FP64 pipe
   if (mcd_ozaki_format(h, M, N, G, &nsl, &rb) != 1 && precision == MCD_PREC_OZAKI_INT8) precision = MCD_PREC_FP64;
   MCD_CUDA(h, cudaSetDevice(h->device));
-  h->last_M = 0;  // whatever was resident is about to be overwritten (also on an early error return)
-  h->last_assign = nullptr;
+  drop_resident(h);  // whatever was resident is about to be overwritten (also on an early error return)
   const int64_t launches0 = h->launches;
   enum { EV_T0 = 0, EV_H2D, EV_STD, EV_CORR, EV_LAPEND, EV_D2H, EV_LAP = 8 };
   const size_t EV_DNA_K1 = 90;  // 2 events around the DNA operand's K1 launch
@@ -1113,10 +1134,7 @@ int mcd_cell2cell_gather(mcd_handle h, const double* rna, int64_t ld_rna, const 
   }
   if (flag) return mcd_fail(h, MCD_ERR_NONFINITE, "NaN or Inf in the expression / copy-number matrix");
   if ((st = step_status(h, bad))) return st;
-  h->last_M = M;
-  h->last_N = N;
-  h->last_ldc = ldc;
-  h->last_assign = out.assign;
+  set_resident(h, M, N, ldc, out.assign);
   return MCD_OK;
 }
 
@@ -1215,8 +1233,8 @@ int mcd_cell2cell_multi(mcd_handle* hs, int ndev, const double* rna, int64_t ld_
       return mcd_fail(h0, MCD_ERR_INVALID, "mcd_cell2cell_multi: gene index out of range");
   int nsl = 0, rb = 0;
   if (mcd_ozaki_format(h0, M, N, G, &nsl, &rb) != 1 && precision == MCD_PREC_OZAKI_INT8) precision = MCD_PREC_FP64;
-  h0->last_M = 0;
-  h0->last_assign = nullptr;
+  // hs[0]'s matrix is about to be overwritten; the other handles' WS_C slots hold shards from now on
+  for (int d = 0; d < ndev; ++d) drop_resident(hs[d]);
   const int64_t ldc = (N + 1) & ~1LL, ldct = (M + 1) & ~1LL;
   const int64_t per = (M + ndev - 1) / ndev;
   const int64_t wr = rna_gene_idx ? ld_rna : G, wd = dna_gene_idx ? ld_dna : G;
@@ -1328,16 +1346,13 @@ int mcd_cell2cell_multi(mcd_handle* hs, int ndev, const double* rna, int64_t ld_
   }
   if (flag) return mcd_fail(h0, MCD_ERR_NONFINITE, "NaN or Inf in the expression / copy-number matrix");
   if ((st = step_status(h0, bad))) return st;
-  h0->last_M = M;
-  h0->last_N = N;
-  h0->last_ldc = ldc;
-  h0->last_assign = out.assign;
+  set_resident(h0, M, N, ldc, out.assign);
   return MCD_OK;
 }
 
 int mcd_corr_rows(mcd_handle h, const int32_t* rows, int64_t nrows, double* out, int out_space) {
   if (!h) return MCD_ERR_INVALID;
-  if (!rows || !out || nrows < 1 || h->last_M < 1 || h->last_assign == nullptr)
+  if (!rows || !out || nrows < 1 || !has_matrix(h))
     return mcd_fail(h, MCD_ERR_INVALID, "mcd_corr_rows: no mcd_cell2cell result is resident");
   for (int64_t i = 0; i < nrows; ++i)
     if (rows[i] < 0 || rows[i] >= h->last_M) return mcd_fail(h, MCD_ERR_INVALID, "mcd_corr_rows: row out of range");
@@ -1365,7 +1380,7 @@ int mcd_corr_rows(mcd_handle h, const int32_t* rows, int64_t nrows, double* out,
 
 int mcd_corr_pairs(mcd_handle h, const int32_t* rows, const int32_t* cols, int64_t n, double* out) {
   if (!h) return MCD_ERR_INVALID;
-  if (!rows || !cols || !out || n < 1 || h->last_M < 1 || h->last_assign == nullptr)
+  if (!rows || !cols || !out || n < 1 || !has_matrix(h))
     return mcd_fail(h, MCD_ERR_INVALID, "mcd_corr_pairs: no mcd_cell2cell result is resident");
   for (int64_t k = 0; k < n; ++k)
     if (rows[k] < 0 || rows[k] >= h->last_M || cols[k] < 0 || cols[k] >= h->last_N)
@@ -1411,7 +1426,7 @@ static int subinstance_steps_impl(mcd_handle h, const int32_t* rna_rows, int64_t
                                   int64_t n_sub, int32_t* assign, int32_t* step, double* step_obj, int out_space,
                                   mcd_stats* stats, bool use_classes, int* bad_out) {
   if (!h) return MCD_ERR_INVALID;
-  if (!assign || !step || m_sub < 1 || n_sub < 1 || h->last_M < 1 || h->last_assign == nullptr)
+  if (!assign || !step || m_sub < 1 || n_sub < 1 || !has_matrix(h))
     return mcd_fail(h, MCD_ERR_INVALID, "mcd_subinstance_steps: no mcd_cell2cell result is resident");
   if ((!rna_rows && m_sub != h->last_M) || (!dna_cols && n_sub != h->last_N))
     return mcd_fail(h, MCD_ERR_INVALID, "mcd_subinstance_steps: NULL index means all rows / columns");
@@ -1500,10 +1515,11 @@ static int sweep_worker(mcd_context* h, size_t k, mcd_context** out) {
   return MCD_OK;
 }
 
-// The replicate sweep engine shared by mcd_subinstance_sweep and mcd_loo_sweep.  Replicates are independent step
-// loops of one shape (m_sub rows, n_sub columns); what makes one replicate differ from the next comes in as hooks.
+// The replicate sweep engine shared by mcd_subinstance_sweep and mcd_loo_sweep and their _multi forms.  Replicates are
+// independent step loops of one shape (m_sub rows, n_sub columns); what makes one replicate differ from the next comes
+// in as hooks.
 struct SweepPlan {
-  int K;              // worker contexts (replicates in flight)
+  int K;              // worker contexts (replicates in flight) per handle
   int64_t nsteps;     // steps of every replicate
   int64_t batch;      // replicates per batch
   size_t step_bytes;  // the replicate's StepOut block (256-byte aligned)
@@ -1524,34 +1540,50 @@ static SweepPlan sweep_plan(int64_t nrep, int64_t m_sub, int64_t n_sub, size_t e
   return p;
 }
 
+// Every hook is called with the handle that owns the batch, h = hs[d], and its index d: a hook reads that handle's
+// resident matrix (its own copy) and that handle's uploads, never another handle's.
 struct SweepHooks {
   // on h->stream before the replicates of the batch [r0, r0 + nb) are dealt (uploads of the batch's indices); optional
-  std::function<int(int64_t r0, int64_t nb)> prepare;
+  std::function<int(mcd_context* h, int d, int64_t r0, int64_t nb)> prepare;
   // on worker w's stream, from w's host thread: cost block subC [m_sub, lds] and its transpose subCt [n_sub, ldst] of
   // replicate r0 + b; *dna_class = DEVICE classes of duplicated DNA cells (see enqueue_step_loop) or NULL
-  std::function<int(mcd_context* w, int64_t r0, int64_t b, double* subC, int64_t lds, double* subCt, int64_t ldst,
-                    const int** dna_class)>
+  std::function<int(mcd_context* h, int d, mcd_context* w, int64_t r0, int64_t b, double* subC, int64_t lds,
+                    double* subCt, int64_t ldst, const int** dna_class)>
       build;
   // on h->stream after the workers joined, before the outputs go to the host: replicate b of the batch has its block
   // at out + b * rep_bytes (StepOut first, the caller's extra bytes from step_bytes on); optional
-  std::function<int(int64_t r0, int64_t nb, char* out)> after;
+  std::function<int(mcd_context* h, int d, int64_t r0, int64_t nb, char* out)> after;
   // on the host once the batch synchronised, per replicate r = r0 + b: status bits and certificate gap in / out (a
-  // replicate may be solved again); optional
-  std::function<int(int64_t r, int64_t b, int& bad, double& gap)> redo;
+  // replicate may be solved again, on h); stats = h's share of the call's stats or NULL; optional
+  std::function<int(mcd_context* h, int d, int64_t r, int64_t b, int& bad, double& gap, mcd_stats* stats)> redo;
 };
 
-static int sweep_replicates(mcd_context* h, const SweepPlan& P, int64_t nrep, int64_t m_sub, int64_t n_sub,
-                            int32_t* assign, int32_t* step, double* step_obj, double* cert_gap, mcd_stats* stats,
-                            const SweepHooks& hk) {
+// What one handle did in a sweep.
+struct SweepShare {
+  int bad = 0;                 // OR of the replicates' status bits
+  double enqueue_ms = 0.0;     // wall time of the enqueuing phases of its batches
+  int64_t launches = 0;        // kernels launched by the handle and its workers
+  int64_t last_r0 = -1;        // first replicate of the last batch it solved
+};
+
+// The batch loop of handle hs[d]: batches [r0, r0 + batch) are claimed from `next_batch` until none is left or `stop`
+// is raised.  With one handle it runs on the caller's thread; with several, each handle has a host thread of its own.
+static int sweep_handle(mcd_context* const* hs, int d, const SweepPlan& P, int64_t batch, int64_t nrep, int64_t m_sub,
+                        int64_t n_sub, int32_t* assign, int32_t* step, double* step_obj, double* cert_gap,
+                        mcd_stats* stats, const SweepHooks& hk, std::atomic<int64_t>& next_batch,
+                        std::atomic<bool>& stop, SweepShare& share) {
+  mcd_context* h = hs[d];
   const int K = P.K;
-  const int64_t nsteps = P.nsteps, batch = P.batch;
+  const int64_t nsteps = P.nsteps;
   const size_t rep_bytes = P.rep_bytes;
   int st;
+  MCD_CUDA(h, cudaSetDevice(h->device));
   void* p_out = nullptr;
   if ((st = mcd_ws(h, WS_SWEEP_OUT, (size_t)batch * rep_bytes, &p_out))) return st;
   const int64_t lds = (n_sub + 1) & ~1LL, ldst = (m_sub + 1) & ~1LL;
   // every worker solves on a slice of the chip: the cooperative grid of the wide rounds is capped so that K of them
-  // are co-resident (the narrow rounds run on one 8- or 16-CTA cluster per solve anyway)
+  // are co-resident (the narrow rounds run on one 8- or 16-CTA cluster per solve anyway).  That slice depends on the
+  // device's SM count and K alone, so a replicate gets the same grid on every device of the same kind.
   std::vector<mcd_context*> ws((size_t)K);
   const int total_blocks = h->sm_count * (h->opt.lap_blocks_per_sm < 1 ? 1 : h->opt.lap_blocks_per_sm);
   for (int k = 0; k < K; ++k) {
@@ -1564,17 +1596,14 @@ static int sweep_replicates(mcd_context* h, const SweepPlan& P, int64_t nrep, in
     }
   }
   const int64_t launches0 = h->launches;
-  // (events 6 / 7 and 8 .. 8 + steps belong to mcd_subinstance_steps, which the class-free re-solve of a replicate runs
-  //  on this handle: the sweep times itself with events of its own)
-  MCD_CUDA(h, cudaEventRecord(get_event(h, 96), h->stream));
   std::vector<mcd_lap_counters> hc((size_t)(nsteps * batch));
   std::vector<mcd_lap_cert> hcert((size_t)(nsteps * batch));
-  if (stats) memset(stats, 0, sizeof *stats);
-  int bad = 0;
-  double host_enqueue_ms = 0.0;  // wall time of the enqueuing phase of every batch: reported as ms_h2d
-  for (int64_t r0 = 0; r0 < nrep; r0 += batch) {
+  for (;;) {
+    if (stop.load()) break;
+    const int64_t r0 = next_batch.fetch_add(1) * batch;
+    if (r0 >= nrep) break;
     const int64_t nb = nrep - r0 < batch ? nrep - r0 : batch;
-    if (hk.prepare && (st = hk.prepare(r0, nb))) return st;
+    if (hk.prepare && (st = hk.prepare(h, d, r0, nb))) return st;
     MCD_CUDA(h, cudaEventRecord(get_event(h, 5), h->stream));
     for (int k = 0; k < K; ++k) MCD_CUDA(h, cudaStreamWaitEvent(ws[k]->stream, get_event(h, 5), 0));
     // Replicates differ a lot in cost (a resampled replicate with a starved clone needs 10x the rounds of a balanced
@@ -1607,7 +1636,7 @@ static int sweep_replicates(mcd_context* h, const SweepPlan& P, int64_t nrep, in
         double* subCt = static_cast<double*>(pct);
         const int* dna_class = nullptr;
         const StepOut out = carve_step_out(static_cast<char*>(p_out) + (size_t)b * rep_bytes, m_sub, nsteps);
-        if ((stw = hk.build(w, r0, b, subC, lds, subCt, ldst, &dna_class)) ||
+        if ((stw = hk.build(h, d, w, r0, b, subC, lds, subCt, ldst, &dna_class)) ||
             (stw = enqueue_step_loop(w, subC, lds, subCt, ldst, m_sub, n_sub, out, 0, false, false, dna_class))) {
           wstatus[(size_t)k] = stw;
           return;
@@ -1629,12 +1658,12 @@ static int sweep_replicates(mcd_context* h, const SweepPlan& P, int64_t nrep, in
     }
     for (int k = 0; k < K; ++k)
       if (wstatus[(size_t)k]) return mcd_fail(h, wstatus[(size_t)k], ws[(size_t)k]->err.c_str());
-    host_enqueue_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - host_t0).count();
+    share.enqueue_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - host_t0).count();
     for (int k = 0; k < K; ++k) {
       MCD_CUDA(h, cudaEventRecord(get_event(ws[k], 0), ws[k]->stream));
       MCD_CUDA(h, cudaStreamWaitEvent(h->stream, get_event(ws[k], 0), 0));
     }
-    if (hk.after && (st = hk.after(r0, nb, static_cast<char*>(p_out)))) return st;
+    if (hk.after && (st = hk.after(h, d, r0, nb, static_cast<char*>(p_out)))) return st;
     // results of the batch: strided device block -> dense host arrays
     const StepOut o0 = carve_step_out(p_out, m_sub, nsteps);
     if (assign)
@@ -1656,32 +1685,164 @@ static int sweep_replicates(mcd_context* h, const SweepPlan& P, int64_t nrep, in
       int bad_b = fold_step_records(h, m_sub, n_sub, nsteps, hc.data() + b * nsteps, rc, stats, 0, false);
       double g = 0.0;
       for (int64_t s2 = 0; s2 < nsteps; ++s2) g = rc[s2].rel_gap > g ? rc[s2].rel_gap : g;
-      if (hk.redo && (st = hk.redo(r0 + b, b, bad_b, g))) return st;
-      bad |= bad_b;
+      if (hk.redo && (st = hk.redo(h, d, r0 + b, b, bad_b, g, stats))) return st;
+      share.bad |= bad_b;
       if (cert_gap) cert_gap[r0 + b] = h->opt.certify ? g : -1.0;
     }
+    if (r0 > share.last_r0) share.last_r0 = r0;
   }
-  MCD_CUDA(h, cudaEventRecord(get_event(h, 97), h->stream));
-  MCD_CUDA(h, cudaStreamSynchronize(h->stream));
-  if (stats) {
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, get_event(h, 96), get_event(h, 97));
-    stats->ms_lap = ms;
-    stats->ms_total = ms;
-    stats->ms_h2d = host_enqueue_ms;
-    stats->n_steps = nsteps;
-    int64_t launches = h->launches - launches0;
-    for (int k = 0; k < K; ++k) launches += ws[k]->launches;
-    stats->kernel_launches = launches;
-  }
-  return step_status(h, bad);
+  share.launches = h->launches - launches0;
+  for (int k = 0; k < K; ++k) share.launches += ws[k]->launches;
+  return MCD_OK;
 }
 
-int mcd_subinstance_sweep(mcd_handle h, int64_t nrep, const int32_t* rna_rows, int64_t m_sub, const int32_t* dna_cols,
-                          int64_t n_sub, int32_t* assign, int32_t* step, double* step_obj, double* cert_gap,
-                          int concurrency, mcd_stats* stats) {
-  if (!h) return MCD_ERR_INVALID;
-  if (!assign || !step || !dna_cols || nrep < 1 || m_sub < 1 || n_sub < 1 || h->last_M < 1 || h->last_assign == nullptr)
+// Replicates [0, nrep) over the handles hs[0..ndev).  One handle: its batch loop on the calling thread, timed with its
+// events.  Several: one host thread per handle, batches claimed from one counter, the solver options of hs[0] on every
+// handle for the duration of the call, stats merged (counters summed, certificate figures the maximum, per-step
+// figures those of the handle that solved the last batch, times the host wall clock of the whole call).
+static int sweep_replicates(mcd_context* const* hs, int ndev, const SweepPlan& P, int64_t nrep, int64_t m_sub,
+                            int64_t n_sub, int32_t* assign, int32_t* step, double* step_obj, double* cert_gap,
+                            mcd_stats* stats, const SweepHooks& hk) {
+  mcd_context* h0 = hs[0];
+  std::atomic<int64_t> next_batch(0);
+  std::atomic<bool> stop(false);
+  if (stats) memset(stats, 0, sizeof *stats);
+  if (ndev == 1) {
+    SweepShare share;
+    MCD_CUDA(h0, cudaSetDevice(h0->device));
+    // (events 6 / 7 and 8 .. 8 + steps belong to mcd_subinstance_steps, which the class-free re-solve of a replicate
+    //  runs on this handle: the sweep times itself with events of its own)
+    MCD_CUDA(h0, cudaEventRecord(get_event(h0, 96), h0->stream));
+    int st = sweep_handle(hs, 0, P, P.batch, nrep, m_sub, n_sub, assign, step, step_obj, cert_gap, stats, hk, next_batch,
+                          stop, share);
+    if (st) return st;
+    MCD_CUDA(h0, cudaEventRecord(get_event(h0, 97), h0->stream));
+    MCD_CUDA(h0, cudaStreamSynchronize(h0->stream));
+    if (stats) {
+      float ms = 0.f;
+      cudaEventElapsedTime(&ms, get_event(h0, 96), get_event(h0, 97));
+      stats->ms_lap = ms;
+      stats->ms_total = ms;
+      stats->ms_h2d = share.enqueue_ms;  // wall time of the enqueuing phase of every batch
+      stats->n_steps = P.nsteps;
+      stats->kernel_launches = share.launches;
+    }
+    return step_status(h0, share.bad);
+  }
+  // Batches small enough that the last ones do not run on one device alone: about four per device
+  // (ceil(nrep / (4 ndev)) replicates), never fewer than the K workers of the device that claims one, never more than
+  // the 1 GiB cap of the plan.
+  int64_t batch = (nrep + 4 * (int64_t)ndev - 1) / (4 * (int64_t)ndev);
+  if (batch < P.K) batch = P.K;
+  if (batch > P.batch) batch = P.batch;
+  std::vector<SweepShare> share((size_t)ndev);
+  std::vector<mcd_stats> dstats((size_t)ndev);
+  std::vector<int> dst((size_t)ndev, MCD_OK);
+  std::vector<mcd_options> saved((size_t)ndev);
+  for (int d = 0; d < ndev; ++d) {
+    memset(&dstats[(size_t)d], 0, sizeof(mcd_stats));
+    saved[(size_t)d] = hs[d]->opt;
+    hs[d]->opt = h0->opt;
+  }
+  const auto t0 = std::chrono::steady_clock::now();
+  auto run = [&](int d) {
+    int st = sweep_handle(hs, d, P, batch, nrep, m_sub, n_sub, assign, step, step_obj, cert_gap,
+                          stats ? &dstats[(size_t)d] : nullptr, hk, next_batch, stop, share[(size_t)d]);
+    if (st == MCD_OK) {
+      const cudaError_t e = cudaStreamSynchronize(hs[d]->stream);
+      if (e != cudaSuccess) st = mcd_fail(hs[d], MCD_ERR_CUDA, "cudaStreamSynchronize", e);
+    }
+    if (st != MCD_OK) stop = true;  // the other handles claim no further batch
+    dst[(size_t)d] = st;
+  };
+  {
+    std::vector<std::thread> threads;
+    for (int d = 1; d < ndev; ++d) threads.emplace_back(run, d);
+    run(0);
+    for (auto& t : threads) t.join();
+  }
+  const double wall_ms = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+  for (int d = 0; d < ndev; ++d) hs[d]->opt = saved[(size_t)d];
+  cudaSetDevice(h0->device);
+  for (int d = 0; d < ndev; ++d)
+    if (dst[(size_t)d] != MCD_OK) return d == 0 ? dst[0] : mcd_fail(h0, dst[(size_t)d], hs[d]->err.c_str());
+  int bad = 0;
+  int last = 0;
+  for (int d = 0; d < ndev; ++d) {
+    bad |= share[(size_t)d].bad;
+    if (share[(size_t)d].last_r0 > share[(size_t)last].last_r0) last = d;
+  }
+  if (stats) {
+    const mcd_stats& L = dstats[(size_t)last];
+    memcpy(stats->step_rounds, L.step_rounds, sizeof L.step_rounds);
+    memcpy(stats->step_bids, L.step_bids, sizeof L.step_bids);
+    memcpy(stats->step_cert_gap, L.step_cert_gap, sizeof L.step_cert_gap);
+    for (int d = 0; d < ndev; ++d) {
+      const mcd_stats& s = dstats[(size_t)d];
+      stats->lap_rounds += s.lap_rounds;
+      stats->lap_bids += s.lap_bids;
+      stats->lap_bytes += s.lap_bytes;
+      stats->lap_aug_rows += s.lap_aug_rows;
+      stats->lap_aug_steps += s.lap_aug_steps;
+      for (int q = 0; q < 8; ++q) stats->lap_cycles[q] += s.lap_cycles[q];
+      stats->cert_bad += s.cert_bad;
+      stats->cert_steps += s.cert_steps;
+      stats->sweep_fallbacks += s.sweep_fallbacks;
+      if (s.cert_rel_gap > stats->cert_rel_gap) stats->cert_rel_gap = s.cert_rel_gap;
+      if (s.cert_max_violation > stats->cert_max_violation) stats->cert_max_violation = s.cert_max_violation;
+      if (share[(size_t)d].enqueue_ms > stats->ms_h2d) stats->ms_h2d = share[(size_t)d].enqueue_ms;
+      stats->kernel_launches += share[(size_t)d].launches;
+    }
+    stats->ms_lap = wall_ms;
+    stats->ms_total = wall_ms;
+    stats->n_steps = P.nsteps;
+  }
+  return step_status(h0, bad);
+}
+
+// Handles of a call: hs[0..ndev) non-NULL and pairwise distinct (one context named twice would be driven by two host
+// threads at once).  Separate contexts on one device are fine.
+static int check_distinct_handles(mcd_context* const* hs, int ndev, const char* what) {
+  char buf[256];
+  for (int d = 0; d < ndev; ++d) {
+    if (!hs[d]) {
+      snprintf(buf, sizeof buf, "%s: handle %d is NULL", what, d);
+      return mcd_fail(hs[0], MCD_ERR_INVALID, buf);
+    }
+    for (int e = 0; e < d; ++e)
+      if (hs[e] == hs[d]) {
+        snprintf(buf, sizeof buf, "%s: handles %d and %d are the same context (a handle may be listed once)", what, e, d);
+        return mcd_fail(hs[0], MCD_ERR_INVALID, buf);
+      }
+  }
+  return MCD_OK;
+}
+
+// Handles of a multi-device view call: distinct, hs[0] holds a resident matrix and every other handle a copy of that
+// same run's matrix (mcd_share_resident since hs[0]'s last run).
+static int check_view_handles(mcd_context* const* hs, int ndev, const char* what) {
+  int st;
+  if ((st = check_distinct_handles(hs, ndev, what))) return st;
+  char buf[320];
+  if (!has_matrix(hs[0])) {
+    snprintf(buf, sizeof buf, "%s: no mcd_cell2cell result is resident on handle 0", what);
+    return mcd_fail(hs[0], MCD_ERR_INVALID, buf);
+  }
+  for (int d = 1; d < ndev; ++d)
+    if (hs[d]->gen != hs[0]->gen || hs[d]->last_M != hs[0]->last_M || hs[d]->last_N != hs[0]->last_N) {
+      snprintf(buf, sizeof buf,
+               "%s: handle %d holds no copy of handle 0's current resident matrix (call mcd_share_resident after "
+               "every run on handle 0)", what, d);
+      return mcd_fail(hs[0], MCD_ERR_INVALID, buf);
+    }
+  return MCD_OK;
+}
+
+static int subinstance_sweep_impl(mcd_context* const* hs, int ndev, int64_t nrep, const int32_t* rna_rows,
+                                  int64_t m_sub, const int32_t* dna_cols, int64_t n_sub, int32_t* assign, int32_t* step,
+                                  double* step_obj, double* cert_gap, int concurrency, mcd_stats* stats) {
+  mcd_context* h = hs[0];
+  if (!assign || !step || !dna_cols || nrep < 1 || m_sub < 1 || n_sub < 1 || !has_matrix(h))
     return mcd_fail(h, MCD_ERR_INVALID, "mcd_subinstance_sweep: no mcd_cell2cell result is resident / bad arguments");
   if (!rna_rows && m_sub != h->last_M)
     return mcd_fail(h, MCD_ERR_INVALID, "mcd_subinstance_sweep: NULL rna_rows means all rows");
@@ -1691,55 +1852,94 @@ int mcd_subinstance_sweep(mcd_handle h, int64_t nrep, const int32_t* rna_rows, i
   for (int64_t j = 0; j < nrep * n_sub; ++j)
     if (dna_cols[j] < 0 || dna_cols[j] >= h->last_N)
       return mcd_fail(h, MCD_ERR_INVALID, "mcd_subinstance_sweep: DNA column out of range");
-  MCD_CUDA(h, cudaSetDevice(h->device));
   const SweepPlan P = sweep_plan(nrep, m_sub, n_sub, 0, concurrency);
   const int64_t batch = P.batch, nsteps = P.nsteps;
-  int st;
-  void* p_idx = nullptr;
-  if ((st = mcd_ws(h, WS_SWEEP_IDX, (size_t)(m_sub + 2 * batch * n_sub) * 4, &p_idx))) return st;
-  int* d_rows = rna_rows ? static_cast<int*>(p_idx) : nullptr;
-  int* d_cols = static_cast<int*>(p_idx) + m_sub;
-  int* d_clss = d_cols + batch * n_sub;
-  std::vector<int> clss((size_t)(batch * n_sub)), cls1;
-  std::vector<int64_t> n_extra((size_t)batch);
-  if (rna_rows) MCD_CUDA(h, cudaMemcpyAsync(d_rows, rna_rows, (size_t)m_sub * 4, cudaMemcpyHostToDevice, h->stream));
-  const double* C = static_cast<const double*>(h->ws[WS_C].ptr);
+  // per handle: the shared RNA rows, the batch's DNA columns and their duplicate classes (device and host)
+  struct Dev {
+    int* d_rows;
+    int* d_cols;
+    int* d_clss;
+    std::vector<int> clss, cls1;
+    std::vector<int64_t> n_extra;
+  };
+  std::vector<Dev> dev((size_t)ndev);
+  for (int d = 0; d < ndev; ++d) {
+    mcd_context* hd = hs[d];
+    Dev& v = dev[(size_t)d];
+    int st;
+    MCD_CUDA(h, cudaSetDevice(hd->device));
+    void* p_idx = nullptr;
+    if ((st = mcd_ws(hd, WS_SWEEP_IDX, (size_t)(m_sub + 2 * batch * n_sub) * 4, &p_idx)))
+      return d == 0 ? st : mcd_fail(h, st, hd->err.c_str());
+    v.d_rows = rna_rows ? static_cast<int*>(p_idx) : nullptr;
+    v.d_cols = static_cast<int*>(p_idx) + m_sub;
+    v.d_clss = v.d_cols + batch * n_sub;
+    v.clss.resize((size_t)(batch * n_sub));
+    v.n_extra.resize((size_t)batch);
+    if (rna_rows)
+      MCD_CUDA(h, cudaMemcpyAsync(v.d_rows, rna_rows, (size_t)m_sub * 4, cudaMemcpyHostToDevice, hd->stream));
+  }
   SweepHooks hk;
-  hk.prepare = [&](int64_t r0, int64_t nb) -> int {
-    MCD_CUDA(h, cudaMemcpyAsync(d_cols, dna_cols + r0 * n_sub, (size_t)nb * n_sub * 4, cudaMemcpyHostToDevice, h->stream));
+  hk.prepare = [&](mcd_context* hd, int d, int64_t r0, int64_t nb) -> int {
+    Dev& v = dev[(size_t)d];
+    MCD_CUDA(hd, cudaMemcpyAsync(v.d_cols, dna_cols + r0 * n_sub, (size_t)nb * n_sub * 4, cudaMemcpyHostToDevice,
+                                 hd->stream));
     for (int64_t b = 0; b < nb; ++b) {
-      n_extra[(size_t)b] = duplicate_classes(dna_cols + (r0 + b) * n_sub, n_sub, cls1);
-      std::copy(cls1.begin(), cls1.end(), clss.begin() + b * n_sub);
+      v.n_extra[(size_t)b] = duplicate_classes(dna_cols + (r0 + b) * n_sub, n_sub, v.cls1);
+      std::copy(v.cls1.begin(), v.cls1.end(), v.clss.begin() + b * n_sub);
     }
-    MCD_CUDA(h, cudaMemcpyAsync(d_clss, clss.data(), (size_t)nb * n_sub * 4, cudaMemcpyHostToDevice, h->stream));
+    MCD_CUDA(hd, cudaMemcpyAsync(v.d_clss, v.clss.data(), (size_t)nb * n_sub * 4, cudaMemcpyHostToDevice, hd->stream));
     return MCD_OK;
   };
-  hk.build = [&](mcd_context* w, int64_t, int64_t b, double* subC, int64_t lds, double* subCt, int64_t ldst,
-                 const int** dna_class) -> int {
+  hk.build = [&](mcd_context* hd, int d, mcd_context* w, int64_t, int64_t b, double* subC, int64_t lds, double* subCt,
+                 int64_t ldst, const int** dna_class) -> int {
+    const Dev& v = dev[(size_t)d];
     dim3 grid((unsigned)((n_sub + 1023) / 1024 < 64 ? (n_sub + 1023) / 1024 : 64), grid_rows(m_sub));
-    gather_sub_kernel<<<grid, 256, 0, w->stream>>>(C, h->last_ldc, d_rows, d_cols + b * n_sub, m_sub, n_sub, subC, lds);
+    gather_sub_kernel<<<grid, 256, 0, w->stream>>>(static_cast<const double*>(hd->ws[WS_C].ptr), hd->last_ldc, v.d_rows,
+                                                   v.d_cols + b * n_sub, m_sub, n_sub, subC, lds);
     MCD_LAUNCH_CHECK(w, "gather_sub_kernel");
-    *dna_class = n_extra[(size_t)b] > 0 ? d_clss + b * n_sub : nullptr;
+    *dna_class = v.n_extra[(size_t)b] > 0 ? v.d_clss + b * n_sub : nullptr;
     return mcd_transpose_f64(w, subC, m_sub, n_sub, lds, subCt, ldst);
   };
-  hk.redo = [&](int64_t r, int64_t b, int& bad_b, double& g) -> int {
-    if (!((bad_b & 2) && n_extra[(size_t)b] > 0)) return MCD_OK;
+  hk.redo = [&](mcd_context* hd, int d, int64_t r, int64_t b, int& bad_b, double& g, mcd_stats* st) -> int {
+    if (!((bad_b & 2) && dev[(size_t)d].n_extra[(size_t)b] > 0)) return MCD_OK;
     // certificate failed with the class treatment of duplicated cells: solve this replicate again without it
     // (see mcd_subinstance_steps)
     mcd_stats st2;
-    const int rc2 = subinstance_steps_impl(h, rna_rows, m_sub, dna_cols + r * n_sub, n_sub, assign + r * m_sub,
+    const int rc2 = subinstance_steps_impl(hd, rna_rows, m_sub, dna_cols + r * n_sub, n_sub, assign + r * m_sub,
                                            step + r * m_sub, step_obj ? step_obj + r * nsteps : nullptr, MCD_MEM_HOST,
                                            &st2, false, &bad_b);
     if (rc2 != MCD_OK && rc2 != MCD_ERR_NOT_CONVERGED) return rc2;
     g = st2.cert_rel_gap;
-    if (stats) stats->sweep_fallbacks += 1;
+    if (st) st->sweep_fallbacks += 1;
     return MCD_OK;
   };
-  return sweep_replicates(h, P, nrep, m_sub, n_sub, assign, step, step_obj, cert_gap, stats, hk);
+  return sweep_replicates(hs, ndev, P, nrep, m_sub, n_sub, assign, step, step_obj, cert_gap, stats, hk);
+}
+
+int mcd_subinstance_sweep(mcd_handle h, int64_t nrep, const int32_t* rna_rows, int64_t m_sub, const int32_t* dna_cols,
+                          int64_t n_sub, int32_t* assign, int32_t* step, double* step_obj, double* cert_gap,
+                          int concurrency, mcd_stats* stats) {
+  if (!h) return MCD_ERR_INVALID;
+  return subinstance_sweep_impl(&h, 1, nrep, rna_rows, m_sub, dna_cols, n_sub, assign, step, step_obj, cert_gap,
+                                concurrency, stats);
+}
+
+int mcd_subinstance_sweep_multi(mcd_handle* hs, int ndev, int64_t nrep, const int32_t* rna_rows, int64_t m_sub,
+                                const int32_t* dna_cols, int64_t n_sub, int32_t* assign, int32_t* step,
+                                double* step_obj, double* cert_gap, int concurrency, mcd_stats* stats) {
+  if (!hs || ndev < 1 || !hs[0]) return MCD_ERR_INVALID;
+  if (ndev == 1)
+    return mcd_subinstance_sweep(hs[0], nrep, rna_rows, m_sub, dna_cols, n_sub, assign, step, step_obj, cert_gap,
+                                 concurrency, stats);
+  int st;
+  if ((st = check_view_handles(hs, ndev, "mcd_subinstance_sweep_multi"))) return st;
+  return subinstance_sweep_impl(hs, ndev, nrep, rna_rows, m_sub, dna_cols, n_sub, assign, step, step_obj, cert_gap,
+                                concurrency, stats);
 }
 
 // Placement of the left-out cells of the replicates [r0, r0 + nb) (blocks at `out`, layout L) and the copies of
-// their results into the dense host outputs.
+// their results into the dense host outputs, on h (its resident matrix, its stream).
 static int loo_place_batch(mcd_context* h, const int* d_cells, int64_t r0, int64_t nb, int64_t m_sub, int64_t nsteps,
                            int64_t k_steps, char* out, const mcd_loo_layout& L, int32_t* test_col, double* test_corr,
                            double* total, double* match_corr) {
@@ -1757,27 +1957,32 @@ static int loo_place_batch(mcd_context* h, const int* d_cells, int64_t r0, int64
   return MCD_OK;
 }
 
-int mcd_loo_sweep(mcd_handle h, const int32_t* cells, int64_t ncells, int64_t k_steps, int32_t* test_col,
-                  double* test_corr, double* total, int32_t* assign, int32_t* step, double* step_obj, double* match_corr,
-                  double* cert_gap, int concurrency, mcd_stats* stats) {
-  if (!h) return MCD_ERR_INVALID;
-  if (h->last_M < 1 || h->last_assign == nullptr)
-    return mcd_fail(h, MCD_ERR_INVALID, "mcd_loo_sweep: no mcd_cell2cell result is resident");
+static int loo_sweep_impl(mcd_context* const* hs, int ndev, const int32_t* cells, int64_t ncells, int64_t k_steps,
+                          int32_t* test_col, double* test_corr, double* total, int32_t* assign, int32_t* step,
+                          double* step_obj, double* match_corr, double* cert_gap, int concurrency, mcd_stats* stats) {
+  mcd_context* h = hs[0];
+  if (!has_matrix(h)) return mcd_fail(h, MCD_ERR_INVALID, "mcd_loo_sweep: no mcd_cell2cell result is resident");
   if (!cells || ncells < 1) return mcd_fail(h, MCD_ERR_INVALID, "mcd_loo_sweep: no cells to leave out");
   if (k_steps < 1) return mcd_fail(h, MCD_ERR_INVALID, "mcd_loo_sweep: k_steps must be >= 1");
   if (!test_col || !test_corr || !total)
     return mcd_fail(h, MCD_ERR_INVALID, "mcd_loo_sweep: test_col, test_corr and total are required");
   for (int64_t r = 0; r < ncells; ++r)
     if (cells[r] < 0 || cells[r] >= h->last_M) return mcd_fail(h, MCD_ERR_INVALID, "mcd_loo_sweep: cell out of range");
-  MCD_CUDA(h, cudaSetDevice(h->device));
   const int64_t N = h->last_N, m_sub = h->last_M - 1;
-  const double* C = static_cast<const double*>(h->ws[WS_C].ptr);
   const int64_t ldc = h->last_ldc;
+  if (m_sub == 0) ndev = 1;  // M == 1: no replicate has a solve; hs[0] places every left-out cell in one launch
+  // per handle: the left-out cells on its device
+  std::vector<const int*> d_cells((size_t)ndev);
   int st;
-  void* p_idx = nullptr;
-  if ((st = mcd_ws(h, WS_SWEEP_IDX, (size_t)ncells * 4, &p_idx))) return st;
-  const int* d_cells = static_cast<const int*>(p_idx);
-  MCD_CUDA(h, cudaMemcpyAsync(p_idx, cells, (size_t)ncells * 4, cudaMemcpyHostToDevice, h->stream));
+  for (int d = 0; d < ndev; ++d) {
+    mcd_context* hd = hs[d];
+    MCD_CUDA(h, cudaSetDevice(hd->device));
+    void* p_idx = nullptr;
+    if ((st = mcd_ws(hd, WS_SWEEP_IDX, (size_t)ncells * 4, &p_idx))) return d == 0 ? st : mcd_fail(h, st, hd->err.c_str());
+    d_cells[(size_t)d] = static_cast<const int*>(p_idx);
+    MCD_CUDA(h, cudaMemcpyAsync(p_idx, cells, (size_t)ncells * 4, cudaMemcpyHostToDevice, hd->stream));
+  }
+  MCD_CUDA(h, cudaSetDevice(h->device));
   // the replicate's extra bytes after its StepOut block: match counts [N], results, matched correlations [m_sub]
   const size_t cnt_bytes = ((size_t)N * 4 + 255) / 256 * 256, res_bytes = 256;
   const size_t mc_bytes = match_corr ? ((size_t)m_sub * 8 + 255) / 256 * 256 : 0;
@@ -1792,7 +1997,7 @@ int mcd_loo_sweep(mcd_handle h, const int32_t* cells, int64_t ncells, int64_t k_
     if ((st = mcd_ws(h, WS_SWEEP_OUT, (size_t)ncells * L.stride, &p_out))) return st;
     const int64_t launches0 = h->launches;
     MCD_CUDA(h, cudaEventRecord(get_event(h, 96), h->stream));
-    if ((st = loo_place_batch(h, d_cells, 0, ncells, 0, 0, k_steps, static_cast<char*>(p_out), L, test_col, test_corr,
+    if ((st = loo_place_batch(h, d_cells[0], 0, ncells, 0, 0, k_steps, static_cast<char*>(p_out), L, test_col, test_corr,
                               total, nullptr)))
       return st;
     MCD_CUDA(h, cudaEventRecord(get_event(h, 97), h->stream));
@@ -1814,24 +2019,48 @@ int mcd_loo_sweep(mcd_handle h, const int32_t* cells, int64_t ncells, int64_t k_
   L.res = P.step_bytes + cnt_bytes;
   L.match = match_corr ? P.step_bytes + cnt_bytes + res_bytes : 0;
   SweepHooks hk;
-  hk.build = [&](mcd_context* w, int64_t r0, int64_t b, double* subC, int64_t lds, double* subCt, int64_t ldst,
-                 const int** dna_class) -> int {
+  hk.build = [&](mcd_context* hd, int, mcd_context* w, int64_t r0, int64_t b, double* subC, int64_t lds, double* subCt,
+                 int64_t ldst, const int** dna_class) -> int {
     *dna_class = nullptr;  // no DNA cell is repeated: the asynchronous solver path
-    int stw = mcd_launch_loo_gather(w, C, ldc, cells[r0 + b], m_sub, N, subC, lds);
+    int stw = mcd_launch_loo_gather(w, static_cast<const double*>(hd->ws[WS_C].ptr), ldc, cells[r0 + b], m_sub, N, subC,
+                                    lds);
     return stw ? stw : mcd_transpose_f64(w, subC, m_sub, N, lds, subCt, ldst);
   };
-  hk.after = [&](int64_t r0, int64_t nb, char* out) -> int {
+  hk.after = [&](mcd_context* hd, int d, int64_t r0, int64_t nb, char* out) -> int {
+    mcd_loo_layout Lb = L;  // a copy per call: the handles' threads run this hook concurrently
     const StepOut o = carve_step_out(out, m_sub, P.nsteps);  // the step loop's outputs inside a replicate's block
-    L.assign = (size_t)(reinterpret_cast<char*>(o.assign) - out);
-    L.obj = (size_t)(reinterpret_cast<char*>(o.obj) - out);
-    return loo_place_batch(h, d_cells, r0, nb, m_sub, P.nsteps, k_steps, out, L, test_col, test_corr, total, match_corr);
+    Lb.assign = (size_t)(reinterpret_cast<char*>(o.assign) - out);
+    Lb.obj = (size_t)(reinterpret_cast<char*>(o.obj) - out);
+    return loo_place_batch(hd, d_cells[(size_t)d], r0, nb, m_sub, P.nsteps, k_steps, out, Lb, test_col, test_corr,
+                           total, match_corr);
   };
-  return sweep_replicates(h, P, ncells, m_sub, N, assign, step, step_obj, cert_gap, stats, hk);
+  return sweep_replicates(hs, ndev, P, ncells, m_sub, N, assign, step, step_obj, cert_gap, stats, hk);
+}
+
+int mcd_loo_sweep(mcd_handle h, const int32_t* cells, int64_t ncells, int64_t k_steps, int32_t* test_col,
+                  double* test_corr, double* total, int32_t* assign, int32_t* step, double* step_obj, double* match_corr,
+                  double* cert_gap, int concurrency, mcd_stats* stats) {
+  if (!h) return MCD_ERR_INVALID;
+  return loo_sweep_impl(&h, 1, cells, ncells, k_steps, test_col, test_corr, total, assign, step, step_obj, match_corr,
+                        cert_gap, concurrency, stats);
+}
+
+int mcd_loo_sweep_multi(mcd_handle* hs, int ndev, const int32_t* cells, int64_t ncells, int64_t k_steps,
+                        int32_t* test_col, double* test_corr, double* total, int32_t* assign, int32_t* step,
+                        double* step_obj, double* match_corr, double* cert_gap, int concurrency, mcd_stats* stats) {
+  if (!hs || ndev < 1 || !hs[0]) return MCD_ERR_INVALID;
+  if (ndev == 1)
+    return mcd_loo_sweep(hs[0], cells, ncells, k_steps, test_col, test_corr, total, assign, step, step_obj, match_corr,
+                         cert_gap, concurrency, stats);
+  int st;
+  if ((st = check_view_handles(hs, ndev, "mcd_loo_sweep_multi"))) return st;
+  return loo_sweep_impl(hs, ndev, cells, ncells, k_steps, test_col, test_corr, total, assign, step, step_obj,
+                        match_corr, cert_gap, concurrency, stats);
 }
 
 int mcd_null_assignments(mcd_handle h, int64_t trials, uint64_t seed, double* sums, double* medians, int out_space) {
   if (!h) return MCD_ERR_INVALID;
-  if (!sums || trials < 1 || h->last_M < 1 || h->last_assign == nullptr)
+  if (!sums || trials < 1 || !has_matrix(h))
     return mcd_fail(h, MCD_ERR_INVALID, "mcd_null_assignments: no mcd_cell2cell result is resident");
   MCD_CUDA(h, cudaSetDevice(h->device));
   double* d_s = sums;
@@ -1844,13 +2073,108 @@ int mcd_null_assignments(mcd_handle h, int64_t trials, uint64_t seed, double* su
     d_m = medians ? d_s + trials : nullptr;
   }
   if ((st = mcd_launch_null_assignments(h, static_cast<const double*>(h->ws[WS_C].ptr), h->last_ldc, h->last_M,
-                                        h->last_N, trials, seed, d_s, d_m)))
+                                        h->last_N, 0, trials, seed, d_s, d_m)))
     return st;
   if (out_space != MCD_MEM_DEVICE) {
     MCD_CUDA(h, cudaMemcpyAsync(sums, d_s, (size_t)trials * 8, cudaMemcpyDeviceToHost, h->stream));
     if (medians) MCD_CUDA(h, cudaMemcpyAsync(medians, d_m, (size_t)trials * 8, cudaMemcpyDeviceToHost, h->stream));
   }
   MCD_CUDA(h, cudaStreamSynchronize(h->stream));
+  return MCD_OK;
+}
+
+int mcd_share_resident(mcd_handle* hs, int ndev) {
+  if (!hs || ndev < 1 || !hs[0]) return MCD_ERR_INVALID;
+  mcd_context* h0 = hs[0];
+  int st;
+  if ((st = check_distinct_handles(hs, ndev, "mcd_share_resident"))) return st;
+  if (!has_matrix(h0)) return mcd_fail(h0, MCD_ERR_INVALID, "mcd_share_resident: no mcd_cell2cell result is resident on handle 0");
+  const size_t bytes = (size_t)h0->last_M * (size_t)h0->last_ldc * 8;
+  const void* src = h0->ws[WS_C].ptr;
+  MCD_CUDA(h0, cudaSetDevice(h0->device));
+  MCD_CUDA(h0, cudaEventRecord(get_event(h0, 95), h0->stream));  // the matrix is complete once this event has passed
+  for (int d = 1; d < ndev; ++d) {
+    mcd_context* h = hs[d];
+    drop_resident(h);  // also if a copy below fails
+    MCD_CUDA(h0, cudaSetDevice(h->device));
+    if (h->device != h0->device) {
+      int can = 0;
+      if (cudaDeviceCanAccessPeer(&can, h->device, h0->device) == cudaSuccess && can) {
+        cudaError_t pe = cudaDeviceEnablePeerAccess(h0->device, 0);
+        if (pe != cudaSuccess) cudaGetLastError();  // already enabled
+      }
+    }
+    void* dst = nullptr;
+    if ((st = mcd_ws(h, WS_C, bytes, &dst))) return mcd_fail(h0, st, h->err.c_str());
+    MCD_CUDA(h0, cudaStreamWaitEvent(h->stream, get_event(h0, 95), 0));
+    if (h->device == h0->device)
+      MCD_CUDA(h0, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, h->stream));
+    else
+      MCD_CUDA(h0, cudaMemcpyPeerAsync(dst, h->device, src, h0->device, bytes, h->stream));
+  }
+  for (int d = 1; d < ndev; ++d) {
+    MCD_CUDA(h0, cudaSetDevice(hs[d]->device));
+    MCD_CUDA(h0, cudaStreamSynchronize(hs[d]->stream));
+  }
+  MCD_CUDA(h0, cudaSetDevice(h0->device));
+  for (int d = 1; d < ndev; ++d) {
+    mcd_context* h = hs[d];
+    h->last_M = h0->last_M;
+    h->last_N = h0->last_N;
+    h->last_ldc = h0->last_ldc;
+    h->last_assign = nullptr;
+    h->gen = h0->gen;
+  }
+  return MCD_OK;
+}
+
+int mcd_null_assignments_multi(mcd_handle* hs, int ndev, int64_t trials, uint64_t seed, double* sums, double* medians) {
+  if (!hs || ndev < 1 || !hs[0]) return MCD_ERR_INVALID;
+  if (ndev == 1) return mcd_null_assignments(hs[0], trials, seed, sums, medians, MCD_MEM_HOST);
+  mcd_context* h0 = hs[0];
+  int st;
+  if ((st = check_view_handles(hs, ndev, "mcd_null_assignments_multi"))) return st;
+  if (!sums || trials < 1) return mcd_fail(h0, MCD_ERR_INVALID, "mcd_null_assignments_multi: bad arguments");
+  // every trial costs the same: handle d takes the contiguous range [lo[d], lo[d + 1]), in proportion to its SMs
+  int64_t sm_total = 0;
+  for (int d = 0; d < ndev; ++d) sm_total += hs[d]->sm_count > 0 ? hs[d]->sm_count : 1;
+  std::vector<int64_t> lo((size_t)ndev + 1);
+  int64_t cum = 0;
+  for (int d = 0; d < ndev; ++d) {
+    lo[(size_t)d] = (int64_t)((__int128)trials * cum / sm_total);
+    cum += hs[d]->sm_count > 0 ? hs[d]->sm_count : 1;
+  }
+  lo[(size_t)ndev] = trials;
+  std::vector<double*> d_s((size_t)ndev, nullptr);
+  for (int d = 0; d < ndev; ++d) {
+    const int64_t n = lo[(size_t)d + 1] - lo[(size_t)d];
+    if (n == 0) continue;
+    mcd_context* h = hs[d];
+    MCD_CUDA(h0, cudaSetDevice(h->device));
+    void* p = nullptr;
+    if ((st = mcd_ws(h, WS_SUB_MISC, (size_t)n * 16, &p))) return d == 0 ? st : mcd_fail(h0, st, h->err.c_str());
+    d_s[(size_t)d] = static_cast<double*>(p);
+    if ((st = mcd_launch_null_assignments(h, static_cast<const double*>(h->ws[WS_C].ptr), h->last_ldc, h->last_M,
+                                          h->last_N, lo[(size_t)d], n, seed, d_s[(size_t)d],
+                                          medians ? d_s[(size_t)d] + n : nullptr)))
+      return d == 0 ? st : mcd_fail(h0, st, h->err.c_str());
+  }
+  // the copies only after every launch: a copy into pageable host memory returns once it is complete
+  for (int d = 0; d < ndev; ++d) {
+    const int64_t n = lo[(size_t)d + 1] - lo[(size_t)d];
+    if (n == 0) continue;
+    mcd_context* h = hs[d];
+    MCD_CUDA(h0, cudaSetDevice(h->device));
+    MCD_CUDA(h0, cudaMemcpyAsync(sums + lo[(size_t)d], d_s[(size_t)d], (size_t)n * 8, cudaMemcpyDeviceToHost, h->stream));
+    if (medians)
+      MCD_CUDA(h0, cudaMemcpyAsync(medians + lo[(size_t)d], d_s[(size_t)d] + n, (size_t)n * 8, cudaMemcpyDeviceToHost,
+                                   h->stream));
+  }
+  for (int d = 0; d < ndev; ++d) {
+    MCD_CUDA(h0, cudaSetDevice(hs[d]->device));
+    MCD_CUDA(h0, cudaStreamSynchronize(hs[d]->stream));
+  }
+  MCD_CUDA(h0, cudaSetDevice(h0->device));
   return MCD_OK;
 }
 

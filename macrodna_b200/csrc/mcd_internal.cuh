@@ -80,7 +80,10 @@ struct mcd_context {
   std::vector<cudaEvent_t> ev;
   // shape of the last mcd_cell2cell call whose correlation matrix / assignment are still resident
   int64_t last_M = 0, last_N = 0, last_ldc = 0;
-  const int* last_assign = nullptr;
+  const int* last_assign = nullptr;  // NULL on a copy (mcd_share_resident): a matrix without an assignment
+  // generation of the resident matrix: a process-wide id given to each successful mcd_cell2cell* run (0 = none); a
+  // copy carries the id of the run it copied, so a multi-device call can tell a current copy from a stale one
+  uint64_t gen = 0;
   // worker contexts of the replicate sweep (own stream + workspace each; same device): replicates are independent
   // problems, and most rounds of a solve keep a handful of SMs busy, so several are kept in flight
   std::vector<mcd_context*> workers;
@@ -173,9 +176,10 @@ int mcd_launch_corr_split(mcd_context* h, const uint16_t* A_hi, const uint16_t* 
                           const uint16_t* B_hi, const uint16_t* B_lo, int64_t N, int64_t ldk16, const double* nA,
                           const double* nB, double* C, int64_t ldc, double* Ct, int64_t ldct);
 
-// Random-assignment null test on a resident correlation matrix (null_test.cu).
-int mcd_launch_null_assignments(mcd_context* h, const double* C, int64_t ldc, int64_t M, int64_t N, int64_t trials,
-                                uint64_t seed, double* d_sums, double* d_medians);
+// Random-assignment null test on a resident correlation matrix (null_test.cu): trials t0 .. t0 + trials - 1, trial
+// t0 + t written at d_sums[t] / d_medians[t].
+int mcd_launch_null_assignments(mcd_context* h, const double* C, int64_t ldc, int64_t M, int64_t N, int64_t t0,
+                                int64_t trials, uint64_t seed, double* d_sums, double* d_medians);
 
 // Leave-one-out sweep (loo.cu).  Byte offsets inside one replicate's block of the sweep's output buffer.
 struct mcd_loo_layout {

@@ -66,15 +66,16 @@ __device__ __forceinline__ double key_f64(unsigned long long k) {
 }
 
 __global__ void __launch_bounds__(NT) null_assign_kernel(const double* __restrict__ C, int64_t ldc, int M, int N, int Mp,
-                                                          int Np, long long trials, unsigned long long seed,
-                                                          double* __restrict__ sums, double* __restrict__ medians) {
+                                                          int Np, long long t0, long long trials,
+                                                          unsigned long long seed, double* __restrict__ sums,
+                                                          double* __restrict__ medians) {
   extern __shared__ unsigned long long nsm[];
   unsigned long long* rk = nsm;        // [Mp] RNA keys -> permutation -> matched values
   unsigned long long* dk = nsm + Mp;   // [Np] DNA keys (last partial step)
   __shared__ double red[NT / 32];
   const int q = M / N, r = M - q * N;
-  for (long long trial = blockIdx.x; trial < trials; trial += gridDim.x) {
-    const unsigned long long base = mix64(seed ^ mix64((unsigned long long)trial));
+  for (long long trial = blockIdx.x; trial < trials; trial += gridDim.x) {  // trial t0 + trial, written at [trial]
+    const unsigned long long base = mix64(seed ^ mix64((unsigned long long)(t0 + trial)));
     for (int i = threadIdx.x; i < Mp; i += NT)
       rk[i] = i < M ? ((mix64(base + 2ull * (unsigned long long)i) >> 13) << 13) | (unsigned long long)i : ~0ull;
     if (r > 0)
@@ -213,7 +214,8 @@ __device__ __forceinline__ unsigned long long* cta_radix_sort(RadixSmem& s, unsi
 
 // One trial at a time per CTA; the CTA's slab of `scratch` holds 2 M keys (+ 2 N when r > 0).  b = index bits.
 __global__ void __launch_bounds__(LNT, 2) null_assign_large_kernel(const double* __restrict__ C, int64_t ldc, int M, int N,
-                                                                int b, long long trials, unsigned long long seed,
+                                                                int b, long long t0, long long trials,
+                                                                unsigned long long seed,
                                                                 unsigned long long* __restrict__ scratch, size_t slab,
                                                                 double* __restrict__ sums, double* __restrict__ medians) {
   __shared__ RadixSmem s;
@@ -224,8 +226,8 @@ __global__ void __launch_bounds__(LNT, 2) null_assign_large_kernel(const double*
   const int q = M / N, r = M - q * N;
   const unsigned long long imask = (1ull << b) - 1ull;
   const int kpass = (64 - b + 7) / 8;  // passes over the hash bits [b, 64)
-  for (long long trial = blockIdx.x; trial < trials; trial += gridDim.x) {
-    const unsigned long long base = mix64(seed ^ mix64((unsigned long long)trial));
+  for (long long trial = blockIdx.x; trial < trials; trial += gridDim.x) {  // trial t0 + trial, written at [trial]
+    const unsigned long long base = mix64(seed ^ mix64((unsigned long long)(t0 + trial)));
     radix_clear(s);
     for (int i = threadIdx.x; i < M; i += LNT) {
       const unsigned long long key = ((mix64(base + 2ull * (unsigned long long)i) >> b) << b) | (unsigned long long)i;
@@ -280,8 +282,8 @@ int pow2_at_least(int64_t n) {
   return p;
 }
 
-int launch_null_large(mcd_context* h, const double* C, int64_t ldc, int64_t M, int64_t N, int64_t trials, uint64_t seed,
-                      double* d_sums, double* d_medians) {
+int launch_null_large(mcd_context* h, const double* C, int64_t ldc, int64_t M, int64_t N, int64_t t0, int64_t trials,
+                      uint64_t seed, double* d_sums, double* d_medians) {
   int b = 13;  // index bits: max(13, bit_length(max(M, N) - 1))
   while (((int64_t)1 << b) < (M > N ? M : N)) ++b;
   const int64_t r = M % N;
@@ -297,7 +299,8 @@ int launch_null_large(mcd_context* h, const double* C, int64_t ldc, int64_t M, i
   void* scratch = nullptr;
   int st;
   if ((st = mcd_ws(h, WS_NULL, (size_t)grid * slab * 8, &scratch))) return st;
-  null_assign_large_kernel<<<(unsigned)grid, LNT, 0, h->stream>>>(C, ldc, (int)M, (int)N, b, (long long)trials,
+  null_assign_large_kernel<<<(unsigned)grid, LNT, 0, h->stream>>>(C, ldc, (int)M, (int)N, b, (long long)t0,
+                                                                 (long long)trials,
                                                                  (unsigned long long)seed,
                                                                  static_cast<unsigned long long*>(scratch), slab,
                                                                  d_sums, d_medians);
@@ -307,12 +310,12 @@ int launch_null_large(mcd_context* h, const double* C, int64_t ldc, int64_t M, i
 
 }  // namespace
 
-int mcd_launch_null_assignments(mcd_context* h, const double* C, int64_t ldc, int64_t M, int64_t N, int64_t trials,
-                                uint64_t seed, double* d_sums, double* d_medians) {
+int mcd_launch_null_assignments(mcd_context* h, const double* C, int64_t ldc, int64_t M, int64_t N, int64_t t0,
+                                int64_t trials, uint64_t seed, double* d_sums, double* d_medians) {
   if (M > NULL_LARGE_MAX || N > NULL_LARGE_MAX)
     return mcd_fail(h, MCD_ERR_UNSUPPORTED,
                     "null test: more than 2^24 cells on a side (fewer than 40 hash bits would remain above the index)");
-  if (M > NULL_MAX || N > NULL_MAX) return launch_null_large(h, C, ldc, M, N, trials, seed, d_sums, d_medians);
+  if (M > NULL_MAX || N > NULL_MAX) return launch_null_large(h, C, ldc, M, N, t0, trials, seed, d_sums, d_medians);
   const int Mp = pow2_at_least(M), Np = pow2_at_least(N);
   const size_t smem = (size_t)(Mp + Np) * 8;
   MCD_CUDA(h, cudaFuncSetAttribute(null_assign_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -321,8 +324,9 @@ int mcd_launch_null_assignments(mcd_context* h, const double* C, int64_t ldc, in
   if (per_sm < 1) per_sm = 1;
   int64_t grid = (int64_t)h->sm_count * per_sm;
   if (grid > trials) grid = trials;
-  null_assign_kernel<<<(unsigned)grid, NT, smem, h->stream>>>(C, ldc, (int)M, (int)N, Mp, Np, (long long)trials,
-                                                              (unsigned long long)seed, d_sums, d_medians);
+  null_assign_kernel<<<(unsigned)grid, NT, smem, h->stream>>>(C, ldc, (int)M, (int)N, Mp, Np, (long long)t0,
+                                                              (long long)trials, (unsigned long long)seed, d_sums,
+                                                              d_medians);
   MCD_LAUNCH_CHECK(h, "null_assign_kernel");
   return MCD_OK;
 }
