@@ -110,7 +110,7 @@ void* mcd_stream(mcd_handle h);
  * same unique optimum on tie-free inputs and redoes a step synchronously when it meets exact ties), "ozaki.slices" (0 = auto),
  * "ozaki.radix" (0 = auto; 128 or 256 forces the digit radix, see mcd_ozaki_format), "ozaki.align", "ozaki.plan", "k1.generic", "k1.no_stream", and the solver knobs "lap.theta", "lap.eps_min", "lap.eps0", "lap.scaling",
  * "lap.max_rounds", "lap.tail_budget", "lap.blocks_per_sm", "lap.grid_blocks", "lap.list_max_m", "lap.lists", "lap.list_min_nu",
- * "lap.tail_cluster", "lap.tail_mh", "lap.tail_sym", "lap.async", "lap.async_nu", "lap.async_threads", "lap.async_blocks_per_sm", "lap.async_stop", "lap.prefetch_rows", "lap.tail_nu", "lap.mh_nu", "lap.scale_cut", "lap.scale_tail_rounds", "lap.scale_full_phases", "lap.aug_nu", "lap.aug_nu_square", "lap.rank_select",
+ * "lap.tail_cluster", "lap.tail_mh", "lap.tail_sym", "lap.async", "lap.async_nu", "lap.async_threads", "lap.async_blocks_per_sm", "lap.async_stop", "lap.sap", "lap.sap_nu", "lap.prefetch_rows", "lap.tail_nu", "lap.mh_nu", "lap.scale_cut", "lap.scale_tail_rounds", "lap.scale_full_phases", "lap.aug_nu", "lap.aug_nu_square", "lap.rank_select",
  * "lap.min_chunk", "lap.chunk_waves".  Unknown names return MCD_ERR_INVALID.
  */
 int mcd_set_option(mcd_handle h, const char* name, double value);

@@ -250,6 +250,8 @@ const OptEntry kOptions[] = {
     MCD_OPT_I("lap.async_threads", lap_async_threads),
     MCD_OPT_I("lap.async_blocks_per_sm", lap_async_blocks_per_sm),
     MCD_OPT_I("lap.async_stop", lap_async_stop),
+    MCD_OPT_I("lap.sap", lap_sap),
+    MCD_OPT_I("lap.sap_nu", lap_sap_nu),
     MCD_OPT_I("lap.prefetch_rows", lap_prefetch_rows),
     MCD_OPT_I("lap.tail_nu", lap_tail_nu),
     MCD_OPT_I("lap.mh_nu", lap_mh_nu),

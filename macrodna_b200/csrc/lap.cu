@@ -118,6 +118,7 @@ struct LapCtrl {
   unsigned long long a_hops;
   int a_tie;       // an exact tie was met (two equal best values, or a bid that cannot raise a price)
   int a_fallback;  // ... so the step is redone by the round-synchronous kernel
+  int sap_cnt[3];  // lap_sap_kernel: frontier lengths of rounds t, t + 1 (being appended) and t + 2 (being cleared)
 };
 
 struct LapState {
@@ -155,6 +156,9 @@ struct LapState {
   int* pred;                 // [m]
   int* sc_col;               // [n + 1] scanned columns in scan order
   double* sc_val;            // [n + 1] their path cost when scanned
+  int* sap_r;                // [2][n] lap_sap_kernel frontier (double buffered by round parity): owner row,
+  double* sap_d;             // [2][n]   distance of the owned column that improved,
+  double* sap_p;             // [2][n]   and the owner's profit
   LapCtrl* ctrl;
   mcd_lap_counters* counters;
   const int* flags;  // [0] != 0: non-finite data was seen upstream -> every solver kernel is a no-op
@@ -2957,6 +2961,261 @@ __global__ void __launch_bounds__(JV_THREADS) lap_augment_kernel(LapState s) {
   }
 }
 
+// ------------------------------------------------------------------------------------------------
+// Phase B on the whole grid (lap.sap): the last lap.sap_nu persons of a rectangular step, handed over by the
+// asynchronous wide kernel.  Dijkstra above pops one column at a time, so a person costs as many dependent row scans
+// as columns it settles (170-290 at 10k x 50k, ~20 us each).  Label-correcting search with pruning needs as many
+// dependent ROUNDS as the shortest-path tree is deep, and a round relaxes all its rows at once:
+//   init   d[j] = -W[f, j] + price[j] (min-form, u_f = 0), pred[j] = f;  best = min over free columns of d
+//   round  the owned columns whose d improved in the last round and is still below best form the frontier; every
+//          column j takes  min over frontier entries (k, r = owner[k]) of ((d[k] - W[r, j]) + profit[r]) + price[j]
+//          (same arithmetic as Dijkstra's relaxation; ties to the smaller row), and keeps it when it is lower than
+//          d[j] by more than GAMMA_TIE -- after the naive auction many persons are exactly indifferent between two
+//          objects, and a cycle of such zero reduced costs that rounds to a few ulps below zero must not be walked
+//          around forever (Dijkstra is protected by its settled set)
+//   stop   when the frontier is empty.  The sink is the free column at best (smaller index on ties: Dijkstra's order),
+//          the JV dual update touches the owned columns below the sink's distance, the path is flipped along pred.
+// Exact from any dual-feasible state, like lap_augment_kernel; the result does not depend on the order of updates.
+// Layout: every CTA owns a fixed slice of the columns and PULLS the frontier rows into it -- each column has one
+// writer, so no atomics on {d, pred}.  One grid barrier per round: a round appends the columns that improved below
+// the previous best, and the next round drops the entries that the fresh best prunes.  scripts/research/sim_lcsap.py
+// is the NumPy restatement (rounds, rows relaxed).
+// ------------------------------------------------------------------------------------------------
+constexpr int SAP_THREADS = 256;
+constexpr int SAP_WARPS = SAP_THREADS / 32;
+constexpr int SAP_UNROLL = 16;  // frontier rows whose W loads one thread has in flight (8 measured the same at C5)
+
+__device__ __forceinline__ bool sap_less(double va, int ja, double vb, int jb) {  // smaller value, then smaller index
+  return (va < vb) | ((va == vb) & (ja < jb));
+}
+// block-wide arg-min of (v, j), returned in every thread
+__device__ __forceinline__ void sap_block_min(double& v, int& j, double* sv, int* sj) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const double ov = __shfl_xor_sync(0xffffffffu, v, o);
+    const int oj = __shfl_xor_sync(0xffffffffu, j, o);
+    if (sap_less(ov, oj, v, j)) v = ov, j = oj;
+  }
+  __syncthreads();  // earlier readers of sv / sj are done
+  if (lane == 0) sv[warp] = v, sj[warp] = j;
+  __syncthreads();
+  v = lane < SAP_WARPS ? sv[lane] : 1.0e300;
+  j = lane < SAP_WARPS ? sj[lane] : 0x7fffffff;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const double ov = __shfl_xor_sync(0xffffffffu, v, o);
+    const int oj = __shfl_xor_sync(0xffffffffu, j, o);
+    if (sap_less(ov, oj, v, j)) v = ov, j = oj;
+  }
+}
+// best free column over the grid: arg-min of the CTAs' partials in slot `slot`; the length of the next frontier is
+// read in the same batch of L2 loads
+__device__ __forceinline__ void sap_grid_min(const LapState& s, int slot, double& v, int& j, double* sv, int* sj,
+                                             const int* cntp, int& cnt) {
+  cnt = cntp != nullptr ? ldm(cntp) : 0;
+  v = 1.0e300;
+  j = 0x7fffffff;
+  for (int q = threadIdx.x; q < (int)gridDim.x; q += SAP_THREADS) {
+    const double qv = ldm(s.pv1 + slot * gridDim.x + q);
+    const int qj = ldm(s.pj1 + slot * gridDim.x + q);
+    if (sap_less(qv, qj, v, j)) v = qv, j = qj;
+  }
+  sap_block_min(v, j, sv, sj);
+}
+
+__global__ void __launch_bounds__(SAP_THREADS) lap_sap_kernel(LapState s) {
+  LapCtrl* ctrl = s.ctrl;
+  // only behind the asynchronous kernel (ascending list of the unassigned persons, exact-CS prices); after an exact
+  // tie the step was redone round-synchronously and its own tail / lap_augment_kernel finish it
+  if (ctrl->finished || !ctrl->in_tail || ctrl->a_fallback || s.flags[0]) return;  // uniform
+  GridBarrier grid{&ctrl->barrier[MAX_PHASES - 3], 0u};  // slots 0 / MAX_PHASES - 1, - 2: the auction kernels
+  __shared__ double sv[SAP_WARPS];
+  __shared__ int sj[SAP_WARPS];
+  __shared__ double e_d[SAP_THREADS], e_p[SAP_THREADS];
+  __shared__ int e_r[SAP_THREADS];
+  __shared__ int e_n;
+  const int tid = threadIdx.x;
+  const int G = gridDim.x;
+  const int m = s.m;
+  const int slice = (m + G - 1) / G;
+  const int j0 = min(m, (int)blockIdx.x * slice), j1 = min(m, j0 + slice);
+  const int waves = (j1 - j0 + SAP_THREADS - 1) / SAP_THREADS;  // uniform over the CTA
+  const int cur_list = ctrl->cur;
+  int* freelist = s.un[cur_list];
+  const int nfree = ctrl->cnt[cur_list];
+  const bool lead = blockIdx.x == 0 && tid == 0;
+  long long rounds = 0, rows = 0;
+  unsigned long long t_init = 0, t_rounds = 0, t_aug = 0, T0, T1, T2, T3;  // (ns, CTA 0)
+  int q = 0, err = 0;  // persons placed; 1 = nothing reachable, 2 = round guard
+  for (; q < nfree; ++q) {
+    if (lead) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(T0));
+    const int f = ldm(freelist + q);
+    if (blockIdx.x == 0 && tid < 3) ctrl->sap_cnt[tid] = 0;
+    // ---- init: distances from f's row, best free column
+    const double* wf = s.W + (int64_t)f * s.ldw;
+    double lv = 1.0e300;
+    int lj = 0x7fffffff;
+    for (int j = j0 + tid; j < j1; j += SAP_THREADS) {
+      const double d = -__ldg(wf + j) + ldm(s.price + j);
+      s.sp[j] = d;
+      s.pred[j] = f;
+      if (ldm(s.owner + j) < 0 && sap_less(d, j, lv, lj)) lv = d, lj = j;
+    }
+    sap_block_min(lv, lj, sv, sj);
+    if (tid == 0) s.pv1[blockIdx.x] = lv, s.pj1[blockIdx.x] = lj;  // slot 0
+    grid.sync();
+    double best;
+    int sink, cnt;
+    sap_grid_min(s, 0, best, sink, sv, sj, nullptr, cnt);
+    if (!(best < 1.0e299)) {  // no free column reachable: only possible on corrupt (non-finite) costs
+      err = 1;
+      break;
+    }
+    for (int j = j0 + tid; j < j1; j += SAP_THREADS) {  // round 0's frontier: every owned column below best
+      const double d = ldm(s.sp + j);
+      const int o = ldm(s.owner + j);
+      if (o >= 0 && d < best) {
+        const int k = atomicAdd(&ctrl->sap_cnt[0], 1);
+        s.sap_r[k] = o;
+        s.sap_d[k] = d;
+        s.sap_p[k] = ldm(s.profit + o);
+      }
+    }
+    grid.sync();
+    cnt = ldm(&ctrl->sap_cnt[0]);
+    if (lead) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(T1));
+    // ---- rounds: round t relaxes list t (buffer t & 1, length sap_cnt[t % 3]) against the best of slot t & 1
+    for (int t = 0;; ++t) {
+      if (cnt == 0) break;
+      if (t > s.n + 1) {  // more rounds than a shortest-path tree can be deep: Dijkstra takes over (exact anyway)
+        err = 2;
+        break;
+      }
+      const int* fr = s.sap_r + (t & 1) * s.n;
+      const double* fd = s.sap_d + (t & 1) * s.n;
+      const double* fp = s.sap_p + (t & 1) * s.n;
+      const int nb = ((t + 1) & 1) * s.n;
+      lv = 1.0e300;
+      lj = 0x7fffffff;
+      for (int wv = 0; wv < waves; ++wv) {
+        const int j = j0 + wv * SAP_THREADS + tid;
+        const bool has = j < j1;
+        // the column's own state is requested up front: nothing in this round changes it before the relaxation ends
+        const double pj = has ? ldm(s.price + j) : 0.0;
+        double d = has ? ldm(s.sp + j) : 0.0;
+        const int o = has ? ldm(s.owner + j) : -1;
+        double bv = 1.0e300;
+        int br = 0x7fffffff;
+        for (int e0 = 0; e0 < cnt; e0 += SAP_THREADS) {
+          __syncthreads();
+          if (tid == 0) e_n = 0;
+          __syncthreads();
+          if (e0 + tid < cnt) {
+            const double dk = ldm(fd + e0 + tid);
+            const double pk = ldm(fp + e0 + tid);
+            const int rk = ldm(fr + e0 + tid);
+            if (dk < best) {  // the fresh best prunes entries appended against the previous one
+              const int k = atomicAdd(&e_n, 1);
+              e_d[k] = dk;
+              e_p[k] = pk;
+              e_r[k] = rk;
+            }
+          }
+          __syncthreads();
+          const int ne = e_n;
+          if (wv == 0) rows += ne;  // (every CTA sees the same frontier: CTA 0 reports it)
+          if (has) {
+            for (int e = 0; e < ne; e += SAP_UNROLL) {
+              double w[SAP_UNROLL];
+#pragma unroll
+              for (int u = 0; u < SAP_UNROLL; ++u)
+                w[u] = e + u < ne ? __ldg(s.W + (int64_t)e_r[e + u] * s.ldw + j) : 0.0;
+#pragma unroll
+              for (int u = 0; u < SAP_UNROLL; ++u) {
+                if (e + u < ne) {
+                  const double v = ((e_d[e + u] - w[u]) + e_p[e + u]) + pj;
+                  if (sap_less(v, e_r[e + u], bv, br)) bv = v, br = e_r[e + u];
+                }
+              }
+            }
+          }
+        }
+        if (has) {
+          if (bv < d - GAMMA_TIE) {
+            d = bv;
+            s.sp[j] = bv;
+            s.pred[j] = br;
+            if (o >= 0 && bv < best) {
+              const int k = atomicAdd(&ctrl->sap_cnt[(t + 1) % 3], 1);
+              s.sap_r[nb + k] = o;
+              s.sap_d[nb + k] = bv;
+              s.sap_p[nb + k] = ldm(s.profit + o);
+            }
+          }
+          if (o < 0 && sap_less(d, j, lv, lj)) lv = d, lj = j;
+        }
+      }
+      sap_block_min(lv, lj, sv, sj);
+      if (tid == 0) s.pv1[((t + 1) & 1) * G + blockIdx.x] = lv, s.pj1[((t + 1) & 1) * G + blockIdx.x] = lj;
+      if (lead) ctrl->sap_cnt[(t + 2) % 3] = 0;  // list t - 1: read before the last barrier
+      grid.sync();
+      sap_grid_min(s, (t + 1) & 1, best, sink, sv, sj, &ctrl->sap_cnt[(t + 1) % 3], cnt);
+      rounds++;
+    }
+    if (err) break;
+    if (lead) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(T2));
+    // ---- JV dual update of the owned columns below the sink's distance, then the augmentation (as lap_augment_kernel)
+    for (int j = j0 + tid; j < j1; j += SAP_THREADS) {
+      const int o = ldm(s.owner + j);
+      const double d = ldm(s.sp + j);
+      if (o >= 0 && d < best) {  // (a person's profit is written by whichever CTA holds its column: through L2)
+        const double dd = best - d;
+        s.price[j] = ldm(s.price + j) + dd;
+        s.profit[o] = ldm(s.profit + o) - dd;
+      }
+    }
+    grid.sync();
+    if (lead) {
+      s.profit[f] = -best;
+      int j = sink;
+      for (int hop = 0;; ++hop) {
+        const int r = ldm(s.pred + j);
+        s.owner[j] = r;
+        const int jn = ldm(s.col4row + r);
+        s.col4row[r] = j;
+        if (r == f || hop > s.n) break;
+        j = jn;
+      }
+    }
+    grid.sync();
+    if (lead) {
+      asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(T3));
+      t_init += T1 - T0, t_rounds += T2 - T1, t_aug += T3 - T2;
+    }
+  }
+  if (lead) {
+    // (ns) distances from the free row, label-correcting rounds, dual update + augmentation; persons placed.  The
+    // master/helper tail's slots: it has nothing to do after this kernel.
+    s.counters->t_phase[4] += (long long)t_init;
+    s.counters->t_phase[5] += (long long)t_rounds;
+    s.counters->t_phase[6] += (long long)t_aug;
+    s.counters->t_phase[7] += q;
+    s.counters->aug_rows += q;
+    s.counters->aug_steps += rounds;
+    s.counters->rounds += rounds;  // dependent grid-wide rounds, like the tail rounds they replace
+    s.counters->bytes += (rows + q) * (long long)m * 8;
+    if (err == 1) s.counters->status |= 1;
+    // round guard: the persons not yet placed go to lap_augment_kernel (the list stays ascending)
+    const int left = err == 2 ? nfree - q : 0;
+    for (int a = 0; a < left; ++a) freelist[a] = freelist[q + a];
+    ctrl->cnt[cur_list] = left;
+    ctrl->stalled = left > 0 ? 1 : 0;
+    ctrl->in_tail = 0;
+    ctrl->finished = 1;
+  }
+}
+
 __global__ void __launch_bounds__(1024) lap_minmax_kernel(const double* __restrict__ W, int n, int m, int64_t ldw,
                                                           LapCtrl* ctrl, int* flags) {
   __shared__ double smin[32], smax[32];
@@ -3243,6 +3502,7 @@ size_t mcd_lap_workspace_bytes(int64_t n, int64_t m) {
   b += align_up(m * 4, 256);            // ocls
   b += align_up(n * 8, 256);            // clevel
   b += align_up(m * 16, 256);           // pw
+  b += align_up(2 * n * 4, 256) + 2 * align_up(2 * n * 8, 256);  // sap_r, sap_d, sap_p
   return b;
 }
 
@@ -3300,6 +3560,9 @@ int mcd_launch_lap(mcd_context* h, const double* W, int64_t n, int64_t m, int64_
   s.ocls = reinterpret_cast<int*>(take(m * 4));
   s.clevel = reinterpret_cast<unsigned long long*>(take(n * 8));
   s.pw = reinterpret_cast<ulonglong2*>(take(m * 16));
+  s.sap_r = reinterpret_cast<int*>(take(2 * n * 4));
+  s.sap_d = reinterpret_cast<double*>(take(2 * n * 8));
+  s.sap_p = reinterpret_cast<double*>(take(2 * n * 8));
   s.pcls = (n < m) ? person_class : nullptr;  // classes ride on the candidate-list bids, which only n < m uses
   s.col4row = col4row;
   s.counters = d_counters;
@@ -3434,6 +3697,21 @@ int mcd_launch_lap(mcd_context* h, const double* W, int64_t n, int64_t m, int64_
       if (opt.lap_grid_blocks > 0 && opt.lap_grid_blocks < async_blocks) async_blocks = opt.lap_grid_blocks;
     }
   }
+  // the asynchronous kernel stops at lap.sap_nu unassigned persons and lap_sap_kernel places them (instead of the
+  // master/helper tail): a grid of one column slice per CTA (at most one 256-column wave each where the chip allows)
+  bool use_sap = use_async && opt.lap_sap != 0;
+  int sap_blocks = 0;
+  if (use_sap) {
+    int sper = 0;
+    MCD_CUDA(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&sper, lap_sap_kernel, SAP_THREADS, 0));
+    sap_blocks = (int)((m + SAP_THREADS - 1) / SAP_THREADS);
+    // more slices than SMs: the same number of CTAs on every SM (a round waits for the most loaded SM)
+    if (sap_blocks > h->sm_count) sap_blocks = (sap_blocks + h->sm_count - 1) / h->sm_count * h->sm_count;
+    if (sap_blocks > h->sm_count * sper) sap_blocks = h->sm_count * sper;
+    if (sap_blocks > MAX_GRID_SLOTS / 2) sap_blocks = MAX_GRID_SLOTS / 2;  // two slots of best-free partials per CTA
+    if (opt.lap_grid_blocks > 0 && opt.lap_grid_blocks < sap_blocks) sap_blocks = opt.lap_grid_blocks;
+    if (sap_blocks < 1) use_sap = false;
+  }
   const int scale_cut_nu = s.scale_cut_nu;
   const long long scale_tail_rounds = s.scale_tail_rounds;
   for (int ph = 0; ph < nphases; ++ph) {
@@ -3446,6 +3724,10 @@ int mcd_launch_lap(mcd_context* h, const double* W, int64_t n, int64_t m, int64_
     if (use_async) {
       int stop_nu = opt.lap_async_stop > 0 && opt.lap_async_stop < tail_nu ? opt.lap_async_stop : tail_nu;
       int max_nu = MH_NU, cont = 0;
+      if (use_sap) {
+        stop_nu = opt.lap_sap_nu > 0 ? opt.lap_sap_nu : 1;
+        if (stop_nu > max_nu) max_nu = stop_nu;
+      }
       if (opt.lap_async_nu > tail_nu) {  // the rounds with more than lap.async_nu bidders stay round-synchronous
         int wide_stop = opt.lap_async_nu, no = 0;
         void* args[] = {&s, &factor, &ph, &wide_stop, &use_lists, &list_min_nu, &aug_nu, &rank_select, &no};
@@ -3461,6 +3743,12 @@ int mcd_launch_lap(mcd_context* h, const double* W, int64_t n, int64_t m, int64_
         int yes = 1;
         void* args[] = {&s, &factor, &ph, &tail_nu, &use_lists, &list_min_nu, &aug_nu, &rank_select, &yes};
         MCD_CUDA(h, cudaLaunchCooperativeKernel((const void*)lap_auction_kernel, dim3(blocks), dim3(LAP_THREADS), args,
+                                                0, h->stream));
+        h->launches++;
+      }
+      if (use_sap) {  // a no-op after the fallback: that step ends in the tail kernels below, as without lap.sap
+        void* sargs[] = {&s};
+        MCD_CUDA(h, cudaLaunchCooperativeKernel((const void*)lap_sap_kernel, dim3(sap_blocks), dim3(SAP_THREADS), sargs,
                                                 0, h->stream));
         h->launches++;
       }

@@ -49,6 +49,8 @@ struct mcd_options {
   int lap_async_threads = 128;  // "lap.async_threads": threads per worker CTA (128 or 256)
   int lap_async_blocks_per_sm = 0;  // "lap.async_blocks_per_sm": 0 = as many as fit
   int lap_async_stop = 8;     // "lap.async_stop": unassigned persons at which the master/helper tail takes over
+  int lap_sap = 1;            // "lap.sap": the asynchronous kernel's last persons go to grid-parallel augmenting paths
+  int lap_sap_nu = 16;        // "lap.sap_nu": ... from this many unassigned persons on (replaces lap.async_stop)
   int lap_tail_nu = -1;       // "lap.tail_nu": -1 = kernel default
   int lap_mh_nu = 32;         // "lap.mh_nu": bidder count at which the master/helper kernel takes over from the wide rounds
   int lap_scale_cut = 0;      // "lap.scale_cut": eps-scaling phases end once at most this many persons still bid
